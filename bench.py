@@ -7,6 +7,9 @@ fp32 |U|^2) plus, for the fwd+adjoint configs, B adjoint propagations (complex64
   python bench.py [--gpus N] [--steps K] [--warmup W] [--config c3]   our CUDA path (default c3 = the headline)
   python bench.py --impl reference ...        the reference's own torch code on the host CPU cores
   python bench.py --impl reference-cuda ...   the reference's own torch code (cuFFT) on the same GPU
+  python bench.py ... --dump-outputs DIR      also write what the last timed step computed as DIR/*.npy
+                                              (rank 0's batch only: with N > 1 GPUs a shard, or one of N batches,
+                                              so compare dumps taken with the same --gpus)
 
   --config  c2    256^2  forward only, B = 4096               (BASELINE.json configs[1])
             c3    1024^2 fwd+adjoint,  B = 512, unpadded      (configs[2], the metric's config; default)
@@ -35,6 +38,7 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
 LAMB, PX = 532e-9, 1.5e-6
+DUMP_LIMIT = 64 * 10**6          # bytes written by --dump-outputs in all
 CONFIGS = {
     # name: field size, batch, padding, adjoint leg, z_max [m], CPU-arm sample (units per step), BASELINE.json config
     "c2": dict(n=256, batch=4096, pad=False, adjoint=False, z_max=1e-3, cpu_units=64,
@@ -230,6 +234,32 @@ def synth(cfg, units, device, seed):
     return O, G, z
 
 
+def dump_outputs(out_dir, arrays, seed=0):
+    """--dump-outputs: write each tensor as out_dir/<name>.npy in float32, complex ones with a trailing (re, im) axis.
+    The tensors share one shape.  When they would take more than DUMP_LIMIT bytes together, each is cut down to the same
+    fixed sample of k distinct flat positions, in increasing order: one position in each of k equal slices of the flat
+    range, drawn by a CPU generator seeded with `seed`.  Equal inputs give identical files from run to run and from
+    build to build."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    numel = next(iter(arrays.values())).numel()
+    assert all(t.numel() == numel for t in arrays.values())
+    per_pos = sum(8 if t.is_complex() else 4 for t in arrays.values())
+    budget = DUMP_LIMIT - 1024 * len(arrays)                 # room for the .npy headers
+    idx = None
+    if numel * per_pos > budget:
+        k = budget // per_pos
+        lo = (torch.arange(k + 1, dtype=torch.float64) * (numel / k)).long()       # slice bounds, lo[k] == numel
+        width = lo[1:] - lo[:-1]                                                    # >= 1 because k < numel
+        off = (torch.rand(k, generator=torch.Generator().manual_seed(seed), dtype=torch.float64) * width).long()
+        idx = lo[:-1] + torch.minimum(off, width - 1)
+    for name, t in arrays.items():
+        x = t if idx is None else t.reshape(-1)[idx.to(t.device)]
+        x = torch.view_as_real(x) if x.is_complex() else x
+        np.save(os.path.join(out_dir, f"{name}.npy"), x.float().cpu().numpy())
+
+
 def cpu_units_per_s(cfg, repeats: int, warmup: int):
     import torch
     orig = getattr(bind_to_gpu_numa_node, "original", None)
@@ -386,6 +416,8 @@ def run_ours(args, cfg):
     ms = float(ms.item())
     clocks = sampler.stop(t0, t1) if rank == 0 else None
     value = total_units * args.steps / (ms * 1e-3)
+    if args.dump_outputs and rank == 0:            # I and A still hold what the last timed step wrote
+        dump_outputs(args.dump_outputs, {"intensity": I, "adjoint": A} if with_adj else {"intensity": I})
 
     # ---- parity spot check of what was just timed: 2 samples of I (and A) against the float64 oracle ----
     parity = None
@@ -578,7 +610,15 @@ def main():
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--no-gpu-baseline", action="store_true")
     ap.add_argument("--bw-test", action="store_true", help="host <-> device copy bandwidth of all ranks at once (names the e2e bound)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write rank 0's outputs of the last step as DIR/intensity.npy and, for "
+                         "the fwd+adjoint configs, DIR/adjoint.npy (float32, adjoint with a trailing (re, im) axis); "
+                         "beyond 64 MB in all, the same fixed, seeded sample of positions of each")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.bw_test):
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     cfg = CONFIGS[args.config]
     if args.impl == "reference":
         return run_reference(args, cfg)

@@ -43,6 +43,25 @@ def test_bench_line_ours():
     assert "workload" in d["config"] and "model" not in d["config"]
 
 
+def test_bench_dump_outputs(tmp_path):
+    """--dump-outputs writes what the last timed step computed; 4 units at 1024^2 fit in 64 MB, so the whole batch is
+    written.  The last unit, which the parity spot check does not look at, against the float64 oracle."""
+    if not torch.cuda.is_available():
+        pytest.skip("needs a CUDA device")
+    import numpy as np
+    import bench
+    from oracle import asm_oracle as ao
+    d = _run("--steps", "2", "--warmup", "3", "--batch", "4", "--no-e2e", "--no-cpu", "--no-gpu-baseline",
+             "--dump-outputs", str(tmp_path))
+    assert d["steps"] == 2
+    i, a = np.load(tmp_path / "intensity.npy"), np.load(tmp_path / "adjoint.npy")
+    assert i.dtype == a.dtype == np.float32 and i.shape == (4, 1, 1024, 1024) and a.shape == (4, 1, 1024, 1024, 2)
+    O, G, z = bench.synth(bench.CONFIGS["c3"], 4, torch.device("cuda"), 1234)
+    o, g, zz = O[3:].cpu().numpy(), G[3:].cpu().numpy(), z[3:].cpu().numpy()
+    assert ao.rel_l2(i[3:], np.abs(ao.asm(o, bench.LAMB, zz, bench.PX)) ** 2) < 1e-4
+    assert ao.rel_l2(a[3:, ..., 0] + 1j * a[3:, ..., 1], ao.asm_adjoint(g, bench.LAMB, zz, bench.PX)) < 1e-4
+
+
 def test_bench_line_reference_arm():
     d = _run("--impl", "reference", "--steps", "1", "--warmup", "0")
     assert d["impl"] == "reference" and d["unit"] == "units/s" and d["value"] > 0
