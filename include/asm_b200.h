@@ -125,6 +125,30 @@ size_t asm_b200_unwrap_workspace_bytes(int B, int H, int W);
 int asm_b200_unwrap(const float* phase, float* out, int B, int H, int W,
                     void* workspace, size_t workspace_bytes, void* stream);
 
+/*
+ * Focal stack: every sample propagated to K distances.  Plane (b, k) equals asm_b200_forward of sample b at distance
+ * z[b*K + k] with C = 1.  The forward row FFT of a sample runs once and is shared by its K planes (its spectrum stays in
+ * the L2-resident workspace); each plane then costs the column pass and the inverse row pass.
+ *   z        : [B][K] distances in metres, z_dtype as in the Conventions (Z_F32: c = fl32(fl32(2 pi) z); Z_F64: 2 pi z).
+ *   in_mode  : IN_COMPLEX, IN_REAL, IN_SQRT_REAL (hologram -> sqrt on load, as Back_prop), IN_AMP_PHASE or
+ *              IN_CONST_AMP_PHASE, with in0 / in1 / in_scale as in asm_b200_forward for C = 1.
+ *   out_mode : OUT_COMPLEX, OUT_INTENSITY or OUT_ABS_ANGLE; out0 (and out1 = angle planes, OUT_ABS_ANGLE only; NULL
+ *              otherwise) are [B][K][N][N].  out0 = NULL: no image output at all (moments only).
+ *   moments  : double [B][K][3] = (Sum |U|, Sum |U|^2, Sum |U|^4) over the N x N output window; overwritten.  NULL: none.
+ *              Reduced from per-row partials in a fixed order (no atomics): repeated calls are bit-identical.
+ * Returns E_NULL if out0 and moments are both NULL; E_SHAPE for B <= 0, K <= 0 or an N / pad that
+ * asm_b200_workspace_bytes rejects; E_MODE for another in/out mode or a non-NULL out1 outside OUT_ABS_ANGLE; otherwise
+ * the codes of the other calls.  Like every call here: stream-ordered on `stream`, no host sync, nothing retained.
+ * asm_b200_focal_stack_workspace_bytes: the workspace it needs (0 = unsupported); never less than
+ * asm_b200_workspace_bytes(B, 1, N, pad), so the same buffer also serves asm_b200_forward of the samples.
+ */
+size_t asm_b200_focal_stack_workspace_bytes(int B, int K, int N, int pad);
+int asm_b200_focal_stack(const void* in0, const void* in1, const void* z, int z_dtype, int K,
+                         void* out0, void* out1, double* moments,
+                         int B, int N, int pad, int in_mode, int out_mode,
+                         double lambda, double px, float in_scale,
+                         void* workspace, size_t workspace_bytes, void* stream);
+
 /* Number of CUDA kernels this library has launched in this process so far (all threads, all devices).
  * Instrumentation for bench.py (`gpu_launches`); not part of the reference's interface. */
 unsigned long long asm_b200_launch_count(void);

@@ -9,6 +9,8 @@ from . import _lib
 from .Angular_Spectrum_Method import ASM, torch_fft, torch_ifft, center_crop
 from .Forward_model import Holo_Generator, Back_prop, unwrap
 from .functional import asm_forward_raw, asm_adjoint_raw, AsmPropagate, HoloIntensity, HoloField
+from .focus import focal_stack, focus_metric, autofocus
 
 __all__ = ["ASM", "Holo_Generator", "Back_prop", "torch_fft", "torch_ifft", "center_crop",
-           "asm_forward_raw", "asm_adjoint_raw", "AsmPropagate", "HoloIntensity", "HoloField", "unwrap"]
+           "asm_forward_raw", "asm_adjoint_raw", "AsmPropagate", "HoloIntensity", "HoloField", "unwrap",
+           "focal_stack", "focus_metric", "autofocus"]

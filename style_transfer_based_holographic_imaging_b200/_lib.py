@@ -16,7 +16,8 @@ ABI_VERSION = 1
 
 SYMBOLS = ["asm_b200_abi_version", "asm_b200_strerror", "asm_b200_workspace_bytes", "asm_b200_forward",
            "asm_b200_adjoint", "asm_b200_grad_z", "asm_b200_launch_count", "asm_b200_profile",
-           "asm_b200_unwrap_workspace_bytes", "asm_b200_unwrap"]
+           "asm_b200_unwrap_workspace_bytes", "asm_b200_unwrap", "asm_b200_focal_stack_workspace_bytes",
+           "asm_b200_focal_stack"]
 
 _lib = None
 
@@ -55,6 +56,10 @@ def load() -> ctypes.CDLL:
     lib.asm_b200_unwrap_workspace_bytes.argtypes = [ci, ci, ci]
     lib.asm_b200_unwrap.restype = ci
     lib.asm_b200_unwrap.argtypes = [vp, vp, ci, ci, ci, vp, sz, vp]
+    lib.asm_b200_focal_stack_workspace_bytes.restype = sz
+    lib.asm_b200_focal_stack_workspace_bytes.argtypes = [ci, ci, ci, ci]
+    lib.asm_b200_focal_stack.restype = ci
+    lib.asm_b200_focal_stack.argtypes = [vp, vp, vp, ci, ci, vp, vp, vp, ci, ci, ci, ci, ci, cd, cd, cf, vp, sz, vp]
     if lib.asm_b200_abi_version() != ABI_VERSION:
         raise AsmB200Error("libasm_b200.so ABI version mismatch; rebuild it")
     _lib = lib

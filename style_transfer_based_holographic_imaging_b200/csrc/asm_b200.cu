@@ -40,7 +40,54 @@ struct Params {
     float in_scale, out_scale, inv_m2;
     int planes, C, N, M, P;               // planes = B*C
     int in_mode, out_mode, aux_mode, h_mode, adj, z_f64;
+    // focal stack (asm_b200_focal_stack): planes are (sample, distance) pairs q = b kst + k.  The column pass reads the
+    // spectrum of sample q / kst from src (slot q / kst - s0) and writes plane q to ws; kst = 0 outside a stack.
+    const float2* src;
+    int kst, s0;
+    double* part;                         // per-row moment partials (Sum |U|, |U|^2, |U|^4) of the planes in ws, or nullptr
 };
+
+// slot of the column pass's source image: in place outside a focal stack, the sample's spectrum inside one
+__device__ __forceinline__ int src_slot(const Params& p, int plane0, int img) { return p.kst ? (plane0 + img) / p.kst - p.s0 : img; }
+__device__ __forceinline__ const float2* src_base(const Params& p) { return p.kst ? p.src : p.ws; }
+
+// Sum |u|, |u|^2, |u|^4 of one value (fp32), accumulated per thread before the row reduction in double
+__device__ __forceinline__ void mom_add(float (&m)[3], float2 u) {
+    const float i2 = fmaf(u.x, u.x, u.y * u.y);
+    m[0] += sqrtf(i2); m[1] += i2; m[2] = fmaf(i2, i2, m[2]);
+}
+// xor-shuffle sum in double over `width` consecutive lanes (a fixed order: repeated calls give identical bits)
+template <int W>
+__device__ __forceinline__ void mom_reduce(double (&d)[3], const float (&m)[3]) {
+#pragma unroll
+    for (int j = 0; j < 3; ++j) d[j] = (double)m[j];
+#pragma unroll
+    for (int o = 1; o < W; o <<= 1) {
+#pragma unroll
+        for (int j = 0; j < 3; ++j) d[j] += __shfl_xor_sync(0xffffffffu, d[j], o);
+    }
+}
+
+// moments[plane0 + i] = Sum of the R row partials of plane i, in index order (one warp per plane)
+__global__ void k_moments_reduce(const double* __restrict__ part, double* __restrict__ mom, int R, int nimg, int plane0) {
+    const int w = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
+    if (w >= nimg) return;
+    double d[3] = {0.0, 0.0, 0.0};
+    const double* src = part + (size_t)w * R * 3;
+    for (int r = lane; r < R; r += 32) {
+#pragma unroll
+        for (int j = 0; j < 3; ++j) d[j] += src[(size_t)r * 3 + j];
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+#pragma unroll
+        for (int j = 0; j < 3; ++j) d[j] += __shfl_xor_sync(0xffffffffu, d[j], o);
+    }
+    if (lane == 0) {
+#pragma unroll
+        for (int j = 0; j < 3; ++j) mom[(size_t)(plane0 + w) * 3 + j] = d[j];
+    }
+}
 
 // phase constant c of a sample (ASM.py:29): fl32(fl32(2 pi) z) for fp32 distances, 2 pi z in double otherwise
 __device__ __forceinline__ double phase_constant_of(const Params& p, int b) {
@@ -305,7 +352,8 @@ __global__ void __launch_bounds__(ROW_THREADS, 1024 / ROW_THREADS) k_rows_fwd(co
     }
 }
 
-template <int n>
+// MOM: also write the focal-stack moment partials (p.part) of the cropped rows
+template <int n, bool MOM = false>
 __global__ void __launch_bounds__(ROW_THREADS, 1024 / ROW_THREADS) k_rows_inv(const Params p, int plane0, int nlines, int ntiles) {
     constexpr int L = 1 << n, TPL = L / 16, LPC = ROW_THREADS / TPL, LP = RowLayout::line_elems(L);
     constexpr TwLayout lay = make_layout(n);
@@ -366,7 +414,7 @@ __global__ void __launch_bounds__(ROW_THREADS, 1024 / ROW_THREADS) k_rows_inv(co
             }
         }
         float dot = 0.f;
-        if (active) {
+        if (active && p.out0) {
             switch (p.out_mode) {
                 case ASM_B200_OUT_COMPLEX: emit16<ASM_B200_OUT_COMPLEX, TPL>(v, p, plane, y, tl, fl, fr); break;
                 case ASM_B200_OUT_INTENSITY: emit16<ASM_B200_OUT_INTENSITY, TPL>(v, p, plane, y, tl, fl, fr); break;
@@ -390,6 +438,24 @@ __global__ void __launch_bounds__(ROW_THREADS, 1024 / ROW_THREADS) k_rows_inv(co
                 if ((t & 31) == 0 && b0 >= 0) atomicAdd((double*)p.out0 + b0, (double)s * K * p.inv_lambda);
             } else if (b >= 0) {
                 atomicAdd((double*)p.out0 + b, (double)dot * K * p.inv_lambda);
+            }
+        }
+        if constexpr (MOM) {
+            // moments of the cropped row: one partial per (row, warp of the row), R = N max(1, TPL / 32) per plane
+            constexpr int W = TPL < 32 ? TPL : 32, WPL = TPL > 32 ? TPL / 32 : 1;
+            float m[3] = {0.f, 0.f, 0.f};
+            if (active) {
+#pragma unroll
+                for (int i = 0; i < 16; ++i) {
+                    const int x = tl + TPL * i - p.P;
+                    if (x >= 0 && x < p.N) mom_add(m, v[i]);
+                }
+            }
+            double d[3];
+            mom_reduce<W>(d, m);
+            if (active && tl % W == 0) {
+                double* dst = p.part + (((size_t)img * p.N + y) * WPL + tl / 32) * 3;
+                dst[0] = d[0]; dst[1] = d[1]; dst[2] = d[2];
             }
         }
         __syncthreads();   // the line buffers (and fold) are reused by the next tile
@@ -416,7 +482,8 @@ __host__ __device__ constexpr int cols_min_blocks(int n) { return n <= 8 ? 4 : n
 
 template <int n>
 __global__ void __launch_bounds__(cols_per_slab(n) * (1 << n) / 16, cols_min_blocks(n))
-k_cols(const Params p, const __grid_constant__ CUtensorMap tmap, const __grid_constant__ CUtensorMap tmap_kz, int plane0) {
+k_cols(const Params p, const __grid_constant__ CUtensorMap tmap, const __grid_constant__ CUtensorMap tmap_src,
+       const __grid_constant__ CUtensorMap tmap_kz, int plane0) {
     constexpr int L = 1 << n, TPL = L / 16, CC = cols_per_slab(n), NT = CC * TPL;
     constexpr bool KZTAB = kz_in_smem(n);            // kappa slab staged in shared memory by TMA
     constexpr bool KZGLOB = use_kz_table(n) && !KZTAB; // kappa read per bin from the global table
@@ -442,7 +509,7 @@ k_cols(const Params p, const __grid_constant__ CUtensorMap tmap, const __grid_co
     if (t == 0) {
         mbar_expect_tx(bar, (uint32_t)(rows * CC * sizeof(float2)) + (KZTAB ? (uint32_t)((L / 2) * CC * sizeof(double)) : 0u));
         for (int r0 = 0; r0 < rows; r0 += boxr)
-            tma_load_3d(slab + (size_t)(p.P + r0) * CC, &tmap, bar, slab_i * CC * 2, r0, img);
+            tma_load_3d(slab + (size_t)(p.P + r0) * CC, &tmap_src, bar, slab_i * CC * 2, r0, src_slot(p, plane0, img));
         if constexpr (KZTAB) {
             for (int r0 = 0; r0 < L / 2; r0 += KBOX)
                 tma_load_3d(kz_s + (size_t)r0 * CC, &tmap_kz, bar, slab_i * CC * 2, r0, 0);
@@ -764,6 +831,7 @@ static cudaError_t set_attrs(size_t smem_fwd, size_t smem_inv, size_t smem_cols)
     cudaError_t e;
     if ((e = set_smem(k_rows_fwd<n>, smem_fwd)) != cudaSuccess) return e;
     if ((e = set_smem(k_rows_inv<n>, smem_inv)) != cudaSuccess) return e;
+    if ((e = set_smem(k_rows_inv<n, true>, smem_inv)) != cudaSuccess) return e;
     if ((e = set_smem(k_cols<n>, smem_cols)) != cudaSuccess) return e;
     attrs_mark(done, dev);
     return cudaSuccess;
@@ -793,7 +861,18 @@ template <class T>
 static void key_add(CallKey& k, const T& v) {
     if (k.len + (int)sizeof(T) <= (int)sizeof(k.b)) { memcpy(k.b + k.len, &v, sizeof(T)); k.len += (int)sizeof(T); }
 }
-static CallKey make_key(const Params& p, const Geometry& g, int kind) {
+// Focal stack (asm_b200_focal_stack): pass 1 of a chunk of samples writes their spectra to S once; then each group of
+// tq planes runs the column pass S -> T and the inverse row pass T -> output (and the moments reduction).  A lane's
+// region is [S: chunk samples][T: tq planes][row moment partials of the tq planes].
+struct StackPlan {
+    int K;                                 // distances per sample
+    int tq;                                // planes per group: a multiple of K (several samples), or <= K (one sample)
+    int R;                                 // moment partials per plane written by the inverse row kernel
+    double* mom;                           // [B][K][3] moments, or nullptr
+    size_t s_elems, t_elems, lane_elems;   // float2 elements of S, T and the whole lane region
+};
+
+static CallKey make_key(const Params& p, const Geometry& g, int kind, const StackPlan* sp) {
     CallKey k;
     memset(&k, 0, sizeof(k));
     key_add(k, p.in0); key_add(k, p.in1); key_add(k, p.aux0); key_add(k, p.aux1); key_add(k, p.out0); key_add(k, p.out1);
@@ -803,6 +882,9 @@ static CallKey make_key(const Params& p, const Geometry& g, int kind) {
     key_add(k, p.planes); key_add(k, p.C); key_add(k, p.N); key_add(k, p.M); key_add(k, p.P);
     key_add(k, p.in_mode); key_add(k, p.out_mode); key_add(k, p.aux_mode); key_add(k, p.h_mode); key_add(k, p.adj); key_add(k, p.z_f64);
     key_add(k, g.n); key_add(k, g.chunk); key_add(k, g.lanes); key_add(k, g.cc); key_add(k, kind);
+    const int stack = sp != nullptr;
+    key_add(k, stack);
+    if (sp) { key_add(k, sp->K); key_add(k, sp->tq); key_add(k, sp->R); key_add(k, sp->mom); key_add(k, sp->lane_elems); }
     return k;
 }
 constexpr int GRAPH_CACHE = 8;
@@ -819,10 +901,12 @@ static GraphCache* graph_cache() {
 // setup(stream) builds the tables; pass(k, lane, stream, params, plane0, nimg) launches pass k of one chunk.
 // A launch error stops the issue loop at the chunk that produced it (the lanes are still joined) and is the call's
 // return value; an error that was already pending when the call started is not attributed to this library.
+// Focal stack (sp != nullptr): a chunk is g.chunk samples; pass 1 writes their spectra to S, then every group of
+// sp->tq planes is 2 launches (3 with moments), so a chunk of c samples costs 1 + c K / tq * (2 or 3) launches.
 template <class Setup, class Pass>
 static int issue_chunks(const Params& p0, const Geometry& g, int L, cudaStream_t st, LaneSet* ls, int lanes, bool prof,
-                        Setup& setup, Pass& pass, unsigned long long* launches_out) {
-    const size_t lane_elems = (size_t)g.chunk * p0.N * L;
+                        Setup& setup, Pass& pass, unsigned long long* launches_out, const StackPlan* sp) {
+    const size_t lane_elems = sp ? sp->lane_elems : (size_t)g.chunk * p0.N * L;
     cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
     if (prof) for (auto& x : ev) cudaEventCreate(&x);
     const cudaError_t pending = cudaPeekAtLastError();
@@ -840,6 +924,33 @@ static int issue_chunks(const Params& p0, const Geometry& g, int L, cudaStream_t
         cudaStream_t s = lanes > 1 ? ls->st[l] : st;
         Params p = p0;
         p.ws = p0.ws + l * lane_elems;
+        if (sp) {
+            if (prof) cudaEventRecord(ev[0], s);
+            pass(0, l, s, p, plane0, nimg);
+            if (prof) cudaEventRecord(ev[1], s);
+            Params pt = p;
+            pt.src = p.ws; pt.ws = p.ws + sp->s_elems; pt.kst = sp->K; pt.s0 = plane0;
+            pt.part = sp->mom ? reinterpret_cast<double*>(pt.ws + sp->t_elems) : nullptr;
+            const int q_end = (plane0 + nimg) * sp->K;
+            for (int q0 = plane0 * sp->K; q0 < q_end; q0 += sp->tq) {
+                const int cnt = q_end - q0 < sp->tq ? q_end - q0 : sp->tq;
+                pass(1, l, s, pt, q0, cnt);
+                pass(2, l, s, pt, q0, cnt);
+                if (pt.part) k_moments_reduce<<<(cnt + 7) / 8, 256, 0, s>>>(pt.part, sp->mom, sp->R, cnt, q0);
+                launches += pt.part ? 3 : 2;
+            }
+            launches += 1;
+            if (pending == cudaSuccess) err = cudaPeekAtLastError();
+            if (prof) {   // the column and inverse row passes of all groups are reported together in the column slot
+                cudaEventRecord(ev[3], s);
+                cudaEventSynchronize(ev[3]);
+                std::lock_guard<std::mutex> lk(g_prof_mu);
+                float ms = 0.f;
+                cudaEventElapsedTime(&ms, ev[0], ev[1]); g_prof_ms[0] += ms;
+                cudaEventElapsedTime(&ms, ev[1], ev[3]); g_prof_ms[1] += ms;
+            }
+            continue;
+        }
         for (int k = 0; k < 3; ++k) {
             if (prof) cudaEventRecord(ev[k], s);
             pass(k, l, s, p, plane0, nimg);
@@ -863,7 +974,8 @@ static int issue_chunks(const Params& p0, const Geometry& g, int L, cudaStream_t
 }
 
 template <class Setup, class Pass>
-static int run_chunks(const Params& p0, const Geometry& g, int L, cudaStream_t st, Setup setup, Pass pass, int kind = 0) {
+static int run_chunks(const Params& p0, const Geometry& g, int L, cudaStream_t st, Setup setup, Pass pass, int kind = 0,
+                      const StackPlan* sp = nullptr) {
     const bool prof = g_profile.load() != 0;
     int lanes = prof ? 1 : g.lanes;
     LaneSet* ls = lanes > 1 ? lanes_for(st) : nullptr;
@@ -880,7 +992,7 @@ static int run_chunks(const Params& p0, const Geometry& g, int L, cudaStream_t s
         if (cudaStreamIsCapturing(st, &cs) != cudaSuccess || cs != cudaStreamCaptureStatusNone) gc = nullptr;   // part of the caller's own graph
     }
     if (gc) {
-        const CallKey key = make_key(p0, g, kind);
+        const CallKey key = make_key(p0, g, kind, sp);
         std::unique_lock<std::mutex> lk(gc->mu);
         GraphEntry* hit = nullptr;
         GraphEntry* victim = &gc->e[0];
@@ -898,7 +1010,7 @@ static int run_chunks(const Params& p0, const Geometry& g, int L, cudaStream_t s
             hit->stamp = ++gc->tick;
             cudaGraph_t graph = nullptr;
             if (cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal) == cudaSuccess) {
-                const int rc = issue_chunks(p0, g, L, st, ls, lanes, false, setup, pass, &launches);
+                const int rc = issue_chunks(p0, g, L, st, ls, lanes, false, setup, pass, &launches, sp);
                 const cudaError_t ec = cudaStreamEndCapture(st, &graph);
                 if (rc == 0 && ec == cudaSuccess && graph && cudaGraphInstantiate(&hit->exec, graph, 0) == cudaSuccess) {
                     cudaGraphDestroy(graph);
@@ -918,13 +1030,13 @@ static int run_chunks(const Params& p0, const Geometry& g, int L, cudaStream_t s
             victim->key = key; victim->seen = 1; victim->launches = 0; victim->stamp = ++gc->tick;
         }
     }
-    const int rc = issue_chunks(p0, g, L, st, ls, lanes, prof, setup, pass, &launches);
+    const int rc = issue_chunks(p0, g, L, st, ls, lanes, prof, setup, pass, &launches, sp);
     g_launches.fetch_add(launches);
     return rc;
 }
 
 template <int n>
-static int launch_n(const Params& p0, const Geometry& g, cudaStream_t st) {
+static int launch_n(const Params& p0, const Geometry& g, cudaStream_t st, const StackPlan* sp = nullptr) {
     constexpr int L = 1 << n, TPL = L / 16, LPC = ROW_THREADS / TPL, CC = cols_per_slab(n);
     constexpr int LP = RowLayout::line_elems(L);
     constexpr TwLayout lay = make_layout(n);
@@ -938,12 +1050,16 @@ static int launch_n(const Params& p0, const Geometry& g, cudaStream_t st) {
 
     EncodeTiledFn enc = get_encode();
     if (!enc) return ASM_B200_E_DRIVER;
-    CUtensorMap tmap[MAX_LANES], tmap_kz;
+    CUtensorMap tmap[MAX_LANES], tmap_t[MAX_LANES], tmap_kz;   // per lane: pass-1 destination, column-pass destination
     const int rows = p0.N;
-    const size_t lane_elems = (size_t)g.chunk * rows * L;
-    for (int l = 0; l < g.lanes; ++l)
+    const size_t lane_elems = sp ? sp->lane_elems : (size_t)g.chunk * rows * L;
+    for (int l = 0; l < g.lanes; ++l) {
         if (!encode3d(enc, &tmap[l], p0.ws + l * lane_elems, 2 * (uint64_t)L, rows, g.chunk, 2 * CC, rows < 256 ? rows : 256))
             return ASM_B200_E_DRIVER;
+        if (!sp) tmap_t[l] = tmap[l];
+        else if (!encode3d(enc, &tmap_t[l], p0.ws + l * lane_elems + sp->s_elems, 2 * (uint64_t)L, rows, sp->tq, 2 * CC, rows < 256 ? rows : 256))
+            return ASM_B200_E_DRIVER;
+    }
     if (kz_in_smem(n)) {
         if (!encode3d(enc, &tmap_kz, const_cast<double*>(p0.kzt), 2 * (uint64_t)L, L / 2, 1, 2 * CC, (L / 2) < 256 ? (L / 2) : 256))
             return ASM_B200_E_DRIVER;
@@ -963,10 +1079,11 @@ static int launch_n(const Params& p0, const Geometry& g, cudaStream_t st) {
         const int ntiles = (nlines + LPC - 1) / LPC;
         const int grid_rows = ntiles < row_ctas_max ? ntiles : row_ctas_max;
         if (k == 0) k_rows_fwd<n><<<grid_rows, ROW_THREADS, smem_fwd, s>>>(p, plane0, nlines, ntiles);
-        else if (k == 1) k_cols<n><<<nimg * (L / CC), CC * TPL, smem_cols, s>>>(p, tmap[lane], tmap_kz, plane0);
+        else if (k == 1) k_cols<n><<<nimg * (L / CC), CC * TPL, smem_cols, s>>>(p, tmap_t[lane], tmap[lane], tmap_kz, plane0);
+        else if (p.part) k_rows_inv<n, true><<<grid_rows, ROW_THREADS, smem_inv, s>>>(p, plane0, nlines, ntiles);
         else k_rows_inv<n><<<grid_rows, ROW_THREADS, smem_inv, s>>>(p, plane0, nlines, ntiles);
     };
-    return run_chunks(p0, g, L, st, setup, pass);
+    return run_chunks(p0, g, L, st, setup, pass, 0, sp);
 }
 
 #ifdef ASM_B200_TUNING
@@ -1188,7 +1305,7 @@ static int launch_32(const Params& p0, const Geometry& g, cudaStream_t st) {
 
 // FFT size 1024, transposed intermediate (k32t.cuh): rows -> tile -> TMA tensor store | warp-private lines | TMA tensor
 // load -> rows.  The workspace of a lane is [chunk][1024 u][N y] complex64, described by one tensor map per lane.
-static int launch_32t(const Params& p0, const Geometry& g, cudaStream_t st) {
+static int launch_32t(const Params& p0, const Geometry& g, cudaStream_t st, const StackPlan* sp = nullptr) {
     constexpr int L = K32_L;
     {
         static std::atomic<unsigned long long> done{0};
@@ -1210,12 +1327,16 @@ static int launch_32t(const Params& p0, const Geometry& g, cudaStream_t st) {
     }
     EncodeTiledFn enc = get_encode();
     if (!enc) return ASM_B200_E_DRIVER;
-    CUtensorMap tmap[MAX_LANES];
-    const size_t lane_elems = (size_t)g.chunk * p0.N * L;
-    for (int l = 0; l < g.lanes; ++l)
-        if (!encode3d(enc, &tmap[l], p0.ws + l * lane_elems, 2 * (uint64_t)p0.N, L, g.chunk, 16, 256, CU_TENSOR_MAP_SWIZZLE_64B,
-                      knob_promo() == 2 ? CU_TENSOR_MAP_L2_PROMOTION_L2_128B : knob_promo() == 1 ? CU_TENSOR_MAP_L2_PROMOTION_L2_64B : CU_TENSOR_MAP_L2_PROMOTION_NONE))
+    CUtensorMap tmap[MAX_LANES], tmap_t[MAX_LANES];                 // per lane: pass-1 destination, pass-3 source
+    const size_t lane_elems = sp ? sp->lane_elems : (size_t)g.chunk * p0.N * L;
+    const CUtensorMapL2promotion promo = knob_promo() == 2 ? CU_TENSOR_MAP_L2_PROMOTION_L2_128B : knob_promo() == 1 ? CU_TENSOR_MAP_L2_PROMOTION_L2_64B : CU_TENSOR_MAP_L2_PROMOTION_NONE;
+    for (int l = 0; l < g.lanes; ++l) {
+        if (!encode3d(enc, &tmap[l], p0.ws + l * lane_elems, 2 * (uint64_t)p0.N, L, g.chunk, 16, 256, CU_TENSOR_MAP_SWIZZLE_64B, promo))
             return ASM_B200_E_DRIVER;
+        if (!sp) tmap_t[l] = tmap[l];
+        else if (!encode3d(enc, &tmap_t[l], p0.ws + l * lane_elems + sp->s_elems, 2 * (uint64_t)p0.N, L, sp->tq, 16, 256, CU_TENSOR_MAP_SWIZZLE_64B, promo))
+            return ASM_B200_E_DRIVER;
+    }
     auto setup = [&](cudaStream_t s) {
         k32t_setup<<<2 * sm_count(), 256, 0, s>>>(const_cast<float2*>(p0.tw), reinterpret_cast<float2*>(const_cast<double*>(p0.kzt)),
                                                   p0.s2, p0.inv_lambda * 0.15915494309189535);
@@ -1231,7 +1352,8 @@ static int launch_32t(const Params& p0, const Geometry& g, cudaStream_t st) {
                               ((p.in_mode == ASM_B200_IN_COMPLEX && in_ok) || (p.in_mode == ASM_B200_IN_AMP_PHASE && in_ok) ||
                                (p.in_mode == ASM_B200_IN_CONST_AMP_PHASE && (p.N % 4 == 0) && ((uintptr_t)p.in1 & 15) == 0));
         const bool inv_bulk = (knob_bulk() & 2) && (p.N % 4 == 0) && ((uintptr_t)p.out0 & 15) == 0 &&
-                              (p.out_mode == ASM_B200_OUT_COMPLEX || (p.out_mode == ASM_B200_OUT_INTENSITY && !p.out1));
+                              (p.out_mode == ASM_B200_OUT_COMPLEX || (p.out_mode == ASM_B200_OUT_INTENSITY && !p.out1)) &&
+                              p.out0 && !p.part;                     // focal-stack moments: the register-store kernel
         if (k == 0) {
             const int in = !fwd_bulk ? 3 : p.in_mode == ASM_B200_IN_COMPLEX ? 0 : p.in_mode == ASM_B200_IN_AMP_PHASE ? 1 : 2;
 #define K32T_FWD(IN) { if (padded) k32t_rows_fwd<IN, true><<<grid_rows, bt, K32T_FWD_SMEM, s>>>(p, tmap[lane], plane0, ngroups); \
@@ -1247,13 +1369,13 @@ static int launch_32t(const Params& p0, const Geometry& g, cudaStream_t st) {
         } else {
             const int out = !inv_bulk ? 2 : p.out_mode == ASM_B200_OUT_INTENSITY ? 1 : 0;
             const int grid_inv = ngroups / 2 < cap_rows ? ngroups / 2 : cap_rows;   // pairs of groups
-#define K32T_INV(OUT) { if (padded) k32t_rows_inv<OUT, true><<<grid_inv, bt, K32T_INV_SMEM, s>>>(p, tmap[lane], plane0, ngroups); \
-                        else k32t_rows_inv<OUT, false><<<grid_inv, bt, K32T_INV_SMEM, s>>>(p, tmap[lane], plane0, ngroups); }
+#define K32T_INV(OUT) { if (padded) k32t_rows_inv<OUT, true><<<grid_inv, bt, K32T_INV_SMEM, s>>>(p, tmap_t[lane], plane0, ngroups); \
+                        else k32t_rows_inv<OUT, false><<<grid_inv, bt, K32T_INV_SMEM, s>>>(p, tmap_t[lane], plane0, ngroups); }
             if (out == 0) K32T_INV(0) else if (out == 1) K32T_INV(1) else K32T_INV(2)
 #undef K32T_INV
         }
     };
-    return run_chunks(p0, g, L, st, setup, pass, 32);
+    return run_chunks(p0, g, L, st, setup, pass, 32, sp);
 }
 
 #ifdef ASM_B200_TUNING
@@ -1263,7 +1385,7 @@ static int launch_64t(const Params& p0, const Geometry& g, cudaStream_t st);
 // FFT size 2048: k64.cuh.  The warp-pair bulk row kernels run when both row passes qualify (complex64 or
 // amplitude / phase in, complex64 or |U|^2 out, 16-byte aligned rows); otherwise the generic row kernels run, with their
 // digit-reversed column order and a kappa table in that order.  The column kernel is the same in both cases.
-static int launch_64(const Params& p0, const Geometry& g, cudaStream_t st) {
+static int launch_64(const Params& p0, const Geometry& g, cudaStream_t st, const StackPlan* sp = nullptr) {
     constexpr int n = 11, L = K64_L, TPL = L / 16, LPC = ROW_THREADS / TPL, LP = RowLayout::line_elems(L);
     constexpr TwLayout lay = make_layout(n);
     const size_t smem_fwd = (size_t)LPC * LP * 8 + (size_t)lay.fwd_end * 8;
@@ -1275,6 +1397,7 @@ static int launch_64(const Params& p0, const Geometry& g, cudaStream_t st) {
             cudaError_t e;
             if ((e = set_smem(k_rows_fwd<n>, smem_fwd)) != cudaSuccess) return (int)e;
             if ((e = set_smem(k_rows_inv<n>, smem_inv)) != cudaSuccess) return (int)e;
+            if ((e = set_smem(k_rows_inv<n, true>, smem_inv)) != cudaSuccess) return (int)e;
             if ((e = set_smem(k64_rows_fwd_bulk<0, false>, K64_ROWS_SMEM)) != cudaSuccess) return (int)e;
             if ((e = set_smem(k64_rows_fwd_bulk<0, true>, K64_ROWS_SMEM)) != cudaSuccess) return (int)e;
             if ((e = set_smem(k64_rows_fwd_bulk<1, false>, K64_ROWS_SMEM)) != cudaSuccess) return (int)e;
@@ -1297,7 +1420,8 @@ static int launch_64(const Params& p0, const Geometry& g, cudaStream_t st) {
     const bool fwd_bulk = (q.in_mode == ASM_B200_IN_COMPLEX && in_ok) || (q.in_mode == ASM_B200_IN_AMP_PHASE && in_ok) ||
                           (q.in_mode == ASM_B200_IN_CONST_AMP_PHASE && (q.N % 4 == 0) && ((uintptr_t)q.in1 & 15) == 0);
     const bool inv_bulk = (q.N % 4 == 0) && ((uintptr_t)q.out0 & 15) == 0 &&
-                          (q.out_mode == ASM_B200_OUT_COMPLEX || (q.out_mode == ASM_B200_OUT_INTENSITY && !q.out1));
+                          (q.out_mode == ASM_B200_OUT_COMPLEX || (q.out_mode == ASM_B200_OUT_INTENSITY && !q.out1)) &&
+                          q.out0 && !(sp && sp->mom);                // focal-stack moments: the generic row kernels
     const bool bulk = fwd_bulk && inv_bulk && knob_bulk() != 0;
 #ifdef ASM_B200_TUNING
     if (bulk && knob_k64t() && q.N % 16 == 0) return launch_64t(p0, g, st);
@@ -1330,6 +1454,7 @@ static int launch_64(const Params& p0, const Geometry& g, cudaStream_t st) {
             const int ntiles = (nlines + LPC - 1) / LPC;
             const int grid_rows = ntiles < row_ctas_max ? ntiles : row_ctas_max;
             if (k == 0) k_rows_fwd<n><<<grid_rows, ROW_THREADS, smem_fwd, s>>>(p, plane0, nlines, ntiles);
+            else if (p.part) k_rows_inv<n, true><<<grid_rows, ROW_THREADS, smem_inv, s>>>(p, plane0, nlines, ntiles);
             else k_rows_inv<n><<<grid_rows, ROW_THREADS, smem_inv, s>>>(p, plane0, nlines, ntiles);
             return;
         }
@@ -1357,11 +1482,12 @@ static int launch_64(const Params& p0, const Geometry& g, cudaStream_t st) {
             }
         }
     };
-    return run_chunks(p0, g, L, st, setup, pass);
+    return run_chunks(p0, g, L, st, setup, pass, 0, sp);
 }
 
-// every even size that is not a power of two: four matrix products (dft_any.cuh), chunks in sequence on the caller's stream
-static int launch_dft(const Params& p0, const DftGeom& g, unsigned char* ws, cudaStream_t st) {
+// every even size that is not a power of two: four matrix products (dft_any.cuh), chunks in sequence on the caller's stream.
+// A focal stack (p0.kst = K) runs the whole transform once per plane (sample q / K), with moments reduced into `mom`.
+static int launch_dft(const Params& p0, const DftGeom& g, unsigned char* ws, cudaStream_t st, double* mom = nullptr) {
     float2* A = reinterpret_cast<float2*>(ws);
     float2* S = reinterpret_cast<float2*>(ws + g.a_bytes);
     float2* T1 = reinterpret_cast<float2*>(ws + g.a_bytes + g.s_bytes);
@@ -1381,6 +1507,10 @@ static int launch_dft(const Params& p0, const DftGeom& g, unsigned char* ws, cud
         k_dft_mm<2><<<dim3(tiles(M), tiles(N), nimg), 256, 0, st>>>(p0, A, S, T1, T2, T3, plane0, N, M);
         k_dft_mm<3><<<dim3(tiles(N), tiles(N), nimg), 256, 0, st>>>(p0, A, S, T1, T2, T3, plane0, N, M);
         launches += 4;
+        if (p0.part) {
+            k_moments_reduce<<<(nimg + 7) / 8, 256, 0, st>>>(p0.part, mom, (int)(tiles(N) * tiles(N)), nimg, plane0);
+            launches += 1;
+        }
         if (pending == cudaSuccess && cudaPeekAtLastError() != cudaSuccess) break;
     }
     g_launches.fetch_add(launches);
@@ -1564,6 +1694,47 @@ extern "C" size_t asm_b200_workspace_bytes(int B, int C, int N, int pad) {
     return dft_geometry(B * C, N, pad, &dg) ? dft_workspace(dg) : 0;
 }
 
+// ---------------------------------------------------------------------------------------------------
+// focal stack
+// ---------------------------------------------------------------------------------------------------
+// Chunking: S (chunk samples) + T (tq planes) + partials of every lane stay within the in-flight budget of a single call,
+// so S is read from L2 by every group of its sample.  The plan depends on (B, K, N, pad) only.
+static bool make_stack_plan(int B, int K, int N, int pad, Geometry* g, StackPlan* sp) {
+    if (B <= 0 || K <= 0 || !make_geometry(B, N, pad, g)) return false;
+    const int n = g->n, M = g->M;
+    int lanes = knob_lanes() != 3 ? knob_lanes() : default_lanes(n, pad != 0);
+    lanes = lanes < 1 ? 1 : (lanes > MAX_LANES ? MAX_LANES : lanes);
+    const size_t budget = knob_chunk_mb() > 0 ? (size_t)knob_chunk_mb() << 20 : default_budget(n, pad != 0);
+    const size_t lane_budget = budget / lanes, img = g->img_bytes;
+    const int R = n == 10 ? N : N * (M / 512 > 1 ? M / 512 : 1);   // partials per plane: k32t_rows_inv / k_rows_inv
+    const size_t per_plane = img + (size_t)R * 3 * sizeof(double);
+    int spc = 1, tq;
+    if (img + (size_t)K * per_plane <= lane_budget) {              // whole stacks of several samples per chunk
+        spc = (int)(lane_budget / (img + (size_t)K * per_plane));
+        if (spc > B) spc = B;
+        tq = spc * K;
+    } else {                                                       // one sample per chunk, its planes in balanced groups
+        const long long gmax = lane_budget > img + per_plane ? (long long)((lane_budget - img) / per_plane) : 1;
+        const long long ng = (K + gmax - 1) / gmax;
+        tq = (int)((K + ng - 1) / ng);
+    }
+    const int nchunks = (B + spc - 1) / spc;
+    if (lanes > nchunks) lanes = nchunks;
+    g->chunk = spc; g->lanes = lanes;
+    sp->K = K; sp->tq = tq; sp->R = R; sp->mom = nullptr;
+    sp->s_elems = (size_t)spc * N * M;
+    sp->t_elems = (size_t)tq * N * M;
+    sp->lane_elems = sp->s_elems + sp->t_elems + align_up((size_t)tq * R * 3, 32);   // doubles, one float2 element each
+    return true;
+}
+static size_t stack_workspace_need(const Geometry& g, const StackPlan& sp) {
+    return g.tw_bytes + g.kz_bytes + sp.lane_elems * sizeof(float2) * g.lanes;
+}
+static size_t dft_stack_partials(const DftGeom& dg) {
+    const size_t t = (size_t)((dg.N + DFT_T - 1) / DFT_T);
+    return align_up((size_t)dg.chunk * t * t * 3 * sizeof(double), 256);
+}
+
 static bool needs_in1(int in_mode) { return in_mode == ASM_B200_IN_AMP_PHASE || in_mode == ASM_B200_IN_COT_FIELD || in_mode == ASM_B200_IN_CONST_AMP_PHASE; }
 
 extern "C" int asm_b200_forward(const void* in0, const void* in1, const void* z, int z_dtype, void* out0, void* out1,
@@ -1676,4 +1847,78 @@ extern "C" int asm_b200_unwrap(const float* phase, float* out, int B, int H, int
         if (e != cudaSuccess) { cudaGetLastError(); return (int)e; }
     }
     return 0;
+}
+
+extern "C" size_t asm_b200_focal_stack_workspace_bytes(int B, int K, int N, int pad) {
+    if (B <= 0 || K <= 0 || (long long)B * K > 0x7fffffffll) return 0;
+    const size_t single = asm_b200_workspace_bytes(B, 1, N, pad);
+    if (!single) return 0;
+    Geometry g;
+    StackPlan sp;
+    DftGeom dg;
+    size_t need;
+    if (make_stack_plan(B, K, N, pad, &g, &sp)) need = stack_workspace_need(g, sp);
+    else if (dft_geometry(B * K, N, pad, &dg)) need = dft_workspace(dg) + dft_stack_partials(dg);
+    else return 0;
+    return need > single ? need : single;   // one buffer also serves asm_b200_forward on the same B, N, pad
+}
+
+extern "C" int asm_b200_focal_stack(const void* in0, const void* in1, const void* z, int z_dtype, int K,
+                                    void* out0, void* out1, double* moments,
+                                    int B, int N, int pad, int in_mode, int out_mode,
+                                    double lambda, double px, float in_scale,
+                                    void* workspace, size_t workspace_bytes, void* stream) {
+    if (!out0 && !moments) return ASM_B200_E_NULL;
+    if (in_mode < 0 || in_mode > ASM_B200_IN_CONST_AMP_PHASE || in_mode == ASM_B200_IN_COT_FIELD) return ASM_B200_E_MODE;
+    if (out_mode != ASM_B200_OUT_COMPLEX && out_mode != ASM_B200_OUT_INTENSITY && out_mode != ASM_B200_OUT_ABS_ANGLE) return ASM_B200_E_MODE;
+    if (out1 && out_mode != ASM_B200_OUT_ABS_ANGLE) return ASM_B200_E_MODE;
+    if (z_dtype != ASM_B200_Z_F32 && z_dtype != ASM_B200_Z_F64) return ASM_B200_E_MODE;
+    if (K <= 0 || B <= 0) return ASM_B200_E_SHAPE;
+    const size_t need = asm_b200_focal_stack_workspace_bytes(B, K, N, pad);
+    if (!need) return ASM_B200_E_SHAPE;
+    if (!(lambda > 0.0) || !(px > 0.0) || !isfinite(lambda) || !isfinite(px)) return ASM_B200_E_OPTICS;
+    if (!workspace || ((uintptr_t)workspace & 255) || workspace_bytes < need) return ASM_B200_E_WORKSPACE;
+    if (!in0 || !z || (needs_in1(in_mode) && !in1)) return ASM_B200_E_NULL;
+    if (out0 && out_mode == ASM_B200_OUT_ABS_ANGLE && !out1) return ASM_B200_E_NULL;
+    int rc = check_device();
+    if (rc) return rc;
+    Params p{};
+    p.in0 = in0; p.in1 = in1; p.out0 = out0; p.out1 = out0 ? out1 : nullptr; p.z = z; p.z_f64 = z_dtype;
+    p.in_mode = in_mode; p.out_mode = out_mode; p.h_mode = H_FWD; p.adj = 0;
+    p.in_scale = in_scale; p.out_scale = 1.f;
+    p.C = 1; p.N = N; p.lambda = lambda; p.inv_lambda = 1.0 / lambda;
+    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+    unsigned char* w = reinterpret_cast<unsigned char*>(workspace);
+    Geometry g;
+    StackPlan sp;
+    if (!make_stack_plan(B, K, N, pad, &g, &sp)) {                   // matrix-product path: one transform per plane
+        DftGeom dg;
+        dft_geometry(B * K, N, pad, &dg);
+        p.planes = B * K; p.M = dg.M; p.P = dg.P; p.kst = K;
+        const double sd = lambda / ((double)dg.M * px);
+        p.s2 = sd * sd;
+        p.inv_m2 = 1.0f / ((float)dg.M * (float)dg.M);
+        p.part = moments ? reinterpret_cast<double*>(w + dft_workspace(dg)) : nullptr;
+        return launch_dft(p, dg, w, st, moments);
+    }
+    sp.mom = moments;
+    p.planes = B; p.M = g.M; p.P = g.P;
+    p.tw = reinterpret_cast<const float2*>(workspace);
+    p.tw32 = p.tw + (g.n == 11 ? make_layout(11).total : 0);
+    p.kzt = g.kz_bytes ? reinterpret_cast<const double*>(w + g.tw_bytes) : nullptr;
+    p.ws = reinterpret_cast<float2*>(w + g.tw_bytes + g.kz_bytes);
+    const double sd = lambda / ((double)g.M * px);
+    p.s2 = sd * sd;
+    p.inv_m2 = 1.0f / ((float)g.M * (float)g.M);
+    switch (g.n) {
+        case 5: return launch_n<5>(p, g, st, &sp);
+        case 6: return launch_n<6>(p, g, st, &sp);
+        case 7: return launch_n<7>(p, g, st, &sp);
+        case 8: return launch_n<8>(p, g, st, &sp);
+        case 9: return launch_n<9>(p, g, st, &sp);
+        case 10: return launch_32t(p, g, st, &sp);
+        case 11: return knob_k64() ? launch_64(p, g, st, &sp) : launch_n<11>(p, g, st, &sp);
+        case 12: return launch_n<12>(p, g, st, &sp);
+    }
+    return ASM_B200_E_SHAPE;
 }

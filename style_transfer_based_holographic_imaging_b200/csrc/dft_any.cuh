@@ -128,7 +128,7 @@ __global__ void __launch_bounds__(256) k_dft_mm(const Params p, const float2* __
             const int rr = e / DFT_K, kk = e % DFT_K, r = r0 + rr, k = k0 + kk;
             float2 val = make_float2(0.f, 0.f);
             if (r < R_ && k < K_) {
-                if (KIND == 0) val = dft_load_any(p, ((size_t)plane * N + r) * N + k);
+                if (KIND == 0) val = dft_load_any(p, ((size_t)(p.kst ? plane / p.kst : plane) * N + r) * N + k);
                 else if (KIND == 1) val = A[(size_t)k * M + r];
                 else if (KIND == 2) val = S[(size_t)k * N + r];
                 else val = T3[((size_t)img * N + r) * M + k];
@@ -172,7 +172,23 @@ __global__ void __launch_bounds__(256) k_dft_mm(const Params p, const float2* __
             const float2 h = dft_h(p, c, r, M, cph);                 // column index = row-pass frequency u, row index = v
             T2[((size_t)img * M + r) * M + c] = make_float2(acc[i].x * h.x - acc[i].y * h.y, acc[i].x * h.y + acc[i].y * h.x);
         } else if (KIND == 2) T3[((size_t)img * N + r) * M + c] = acc[i];
-        else dot += dft_emit_any(p, plane, r, c, acc[i]);
+        else if (p.out0) dot += dft_emit_any(p, plane, r, c, acc[i]);
+    }
+    if (KIND == 3 && p.part) {                                       // focal-stack moments: one partial per tile, fixed order
+        float m[3] = {0.f, 0.f, 0.f};
+#pragma unroll
+        for (int i = 0; i < 4; ++i)
+            if (r0 + ty + 8 * i < N && c < N) mom_add(m, acc[i]);
+        double d[3];
+        mom_reduce<32>(d, m);
+        __shared__ double mred[8][3];
+        if ((t & 31) == 0) { mred[t >> 5][0] = d[0]; mred[t >> 5][1] = d[1]; mred[t >> 5][2] = d[2]; }
+        __syncthreads();
+        if (t < 3) {
+            double s = 0.0;
+            for (int w = 0; w < 8; ++w) s += mred[w][t];
+            p.part[(((size_t)img * gridDim.y + blockIdx.y) * gridDim.x + blockIdx.x) * 3 + t] = s;
+        }
     }
     if (KIND == 3 && p.out_mode == OUT_DOT) {                        // uniform branch: reduce the block, one atomic
 #pragma unroll

@@ -268,7 +268,8 @@ __global__ void __launch_bounds__(32 * K32T_LINE_WARPS, K32T_LINE_CTAS) k32t_lin
     auto request = [&](int line, bool with_kappa) {                  // lane 0 only
         const int u = line & 1023, ru = u <= 512 ? u : 1024 - u;
         mbar_expect_tx(bar, (unsigned)N * 8u + (with_kappa ? KAP_ROW_B : 0u));
-        bulk_load(xch, p.ws + (size_t)line * N, (unsigned)N * 8u, bar, pol);
+        const size_t src_line = ((size_t)src_slot(p, plane0, line >> 10) << 10) | (unsigned)(line & 1023);
+        bulk_load(xch, src_base(p) + src_line * N, (unsigned)N * 8u, bar, pol);
         if (with_kappa) bulk_load(kap_s, kap2 + (size_t)ru * KAP_STRIDE, KAP_ROW_B, bar, pol);
     };
     const int nwarps = gridDim.x * K32T_LINE_WARPS, wg = blockIdx.x * K32T_LINE_WARPS + w;
@@ -425,7 +426,7 @@ k32t_rows_inv(const Params p, const __grid_constant__ CUtensorMap tmapT, int pla
         }
         if constexpr (OUT == 2) {
             float dot = 0.f;
-            switch (p.out_mode) {
+            if (p.out0) switch (p.out_mode) {
                 case ASM_B200_OUT_COMPLEX: emit32<ASM_B200_OUT_COMPLEX>(v, p, plane, y, lane, fl, fr); break;
                 case ASM_B200_OUT_INTENSITY: emit32<ASM_B200_OUT_INTENSITY>(v, p, plane, y, lane, fl, fr); break;
                 case ASM_B200_OUT_ABS_ANGLE: emit32<ASM_B200_OUT_ABS_ANGLE>(v, p, plane, y, lane, fl, fr); break;
@@ -439,6 +440,20 @@ k32t_rows_inv(const Params p, const __grid_constant__ CUtensorMap tmapT, int pla
                 for (int o = 16; o > 0; o >>= 1) dot += __shfl_xor_sync(0xffffffffu, dot, o);
                 const double K = p.z_f64 ? 6.283185307179586 : (double)6.2831854820251465f;
                 if (lane == 0) atomicAdd((double*)p.out0 + plane / p.C, (double)dot * K * p.inv_lambda);
+            }
+            if (p.part) {                                            // moments of the cropped row: one partial per row
+                float m[3] = {0.f, 0.f, 0.f};
+#pragma unroll
+                for (int i = 0; i < 32; ++i) {
+                    const int x = lane + 32 * i - (PADDED ? p.P : 0);
+                    if (x >= 0 && x < N) mom_add(m, v[i]);
+                }
+                double d[3];
+                mom_reduce<32>(d, m);
+                if (lane == 0) {
+                    double* dst = p.part + ((size_t)img * N + y) * 3;
+                    dst[0] = d[0]; dst[1] = d[1]; dst[2] = d[2];
+                }
             }
             fence_proxy_async();                                     // the line reads are done before the next tile lands on them
         } else {

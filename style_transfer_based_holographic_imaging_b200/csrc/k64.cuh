@@ -330,7 +330,7 @@ __global__ void __launch_bounds__(64 * K64_CC, 2) k64_cols(const Params p, int p
     for (int i = t; i < K32_TW; i += 64 * CC) tw[i] = __ldg(p.tw32 + i);
     int wi = blockIdx.x;
     if (wi < total) {
-        k64_stage_raw(raw, p.ws + (size_t)(wi / nslab) * N * L, (wi % nslab) * CC, N);
+        k64_stage_raw(raw, src_base(p) + (size_t)src_slot(p, plane0, wi / nslab) * N * L, (wi % nslab) * CC, N);
         k64_stage_kz(kz_s, p.kzt, (wi % nslab) * CC);
         cp_async_commit();
     }
@@ -437,7 +437,7 @@ __global__ void __launch_bounds__(64 * K64_CC, 2) k64_cols(const Params p, int p
             v[i] = h == 0 ? make_float2(v[i].x + o.x, v[i].y + o.y) : make_float2(o.x - v[i].x, o.y - v[i].y);   // row 1024 h + tl + 32 i
         }
         __syncthreads();                                             // the slabs are dead: land the next item in them
-        if (nxt < total) k64_stage_raw(raw, p.ws + (size_t)(nxt / nslab) * N * L, (nxt % nslab) * CC, N);
+        if (nxt < total) k64_stage_raw(raw, src_base(p) + (size_t)src_slot(p, plane0, nxt / nslab) * N * L, (nxt % nslab) * CC, N);
         cp_async_commit();
         // ---- store rows [P, P+N) (crop); adjoint: fold the padding rows onto rows P and P+N-1 first ----
         float2* dst = img_ws + col0 + c;
