@@ -252,6 +252,162 @@ def holo_generator_vjp(amplitude, phase, d, w, args):
     return grad_a, grad_phi, grad_d
 
 
+# --------------------------------------------------------------------------------------------
+# the C ABI's modes (include/asm_b200.h), the transfer function on its own, and a complex64 pipeline
+# --------------------------------------------------------------------------------------------
+IN_COMPLEX, IN_AMP_PHASE, IN_SQRT_REAL, IN_COT_FIELD, IN_REAL, IN_CONST_AMP_PHASE = range(6)
+OUT_COMPLEX, OUT_INTENSITY, OUT_ABS_ANGLE, OUT_REIM_CAT, OUT_ABSANG_CAT, OUT_GRAD_AP = range(6)
+
+
+def transfer_function(m: int, n: int, lamb: float, px: float, d) -> np.ndarray:
+    """H = exp(i c kz) on the unshifted m x m bins, one table per distance: [len(d), m, m] complex128.
+
+    ``kz_unshifted`` (evanescent bins clamped to kz = 0, so H = 1 there) times ``phase_constant(d)``.
+    """
+    kz = kz_unshifted(m, n, lamb, px)
+    c = phase_constant(np.atleast_1d(d))
+    return np.exp(1j * (c[:, None, None] * kz[None]))
+
+
+def grad_constant(d) -> float:
+    """K of dU/dz = ifft2(i K kz H fft2(O)): fl32(2 pi) for fp32 distances, 2 pi for fp64 ones."""
+    return float(TWO_PI_F32) if np.asarray(d).dtype == np.float32 else 2.0 * np.pi
+
+
+def scaled_phase(phase, in_scale) -> np.ndarray:
+    """``fl32(phase * in_scale)`` as float64: the phase the library takes sin / cos of."""
+    return (np.asarray(phase, dtype=np.float32) * np.float32(in_scale)).astype(np.float32).astype(np.float64)
+
+
+def input_field(in_mode: int, in0, in1=None, in_scale: float = 1.0) -> np.ndarray:
+    """The complex128 field O that ``in_mode`` builds from (in0, in1) (include/asm_b200.h, IN_*)."""
+    if in_mode == IN_COMPLEX:
+        return np.asarray(in0).astype(np.complex128)
+    if in_mode == IN_AMP_PHASE:
+        return np.asarray(in0, dtype=np.float64) * np.exp(1j * scaled_phase(in1, in_scale))
+    if in_mode == IN_CONST_AMP_PHASE:
+        return float(np.asarray(in0).reshape(-1)[0]) * np.exp(1j * scaled_phase(in1, in_scale))
+    if in_mode == IN_SQRT_REAL:
+        return np.sqrt(np.asarray(in0, dtype=np.float64)).astype(np.complex128)
+    if in_mode == IN_COT_FIELD:
+        return 2.0 * np.asarray(in0, dtype=np.float64) * np.asarray(in1).astype(np.complex128)
+    if in_mode == IN_REAL:
+        return np.asarray(in0, dtype=np.float64).astype(np.complex128)
+    raise ValueError(f"unknown in_mode {in_mode}")
+
+
+def _fft_pair(dtype=np.complex128):
+    """(fft2, ifft2) over the last two axes: scipy.fft keeps complex128 in double and complex64 in single precision."""
+    import scipy.fft as sf
+    return (lambda x: sf.fft2(x, workers=-1)), (lambda x: sf.ifft2(x, workers=-1))
+
+
+def propagate_h(o: np.ndarray, h: np.ndarray, zero_padding: bool = False, adjoint: bool = False,
+                dtype=np.complex128) -> np.ndarray:
+    """The library's operator with an explicit transfer function ``h`` (broadcast against [B,C,M,M]).
+
+    forward: crop(ifft2(h fft2(replicate_pad(o))));  adjoint: replicate_pad^T(ifft2(conj(h) fft2(zero_embed(o)))).
+    ``dtype`` complex64 runs both transforms in single precision with ``h`` rounded to complex64.
+    """
+    fft2, ifft2 = _fft_pair(dtype)
+    o = np.asarray(o)
+    b, ch, n, _ = o.shape
+    m = 2 * n if zero_padding else n
+    p = (m - n) // 2
+    h = np.asarray(h).astype(dtype)
+    if adjoint:
+        x = np.zeros((b, ch, m, m), dtype=dtype)
+        x[:, :, p:p + n, p:p + n] = o
+        y = ifft2(np.conj(h) * fft2(x)).astype(dtype)
+        return replicate_pad_T(y, n, p) if p else y
+    idx = np.clip(np.arange(m) - p, 0, n - 1)
+    x = o.astype(dtype)[:, :, idx][:, :, :, idx]
+    return ifft2(h * fft2(x)).astype(dtype)[:, :, p:p + n, p:p + n]
+
+
+def _h_per_sample(n: int, zero_padding: bool, lamb: float, d, px: float, batch: int) -> np.ndarray:
+    m = 2 * n if zero_padding else n
+    return transfer_function(m, n, lamb, px, _as_b(d, batch))[:, None]
+
+
+def asm_c128(o, lamb, d, px, zero_padding=False, adjoint=False) -> np.ndarray:
+    """Forward (``asm_closed_form``) or exact adjoint (``asm_adjoint``) through ``propagate_h`` in float64."""
+    o = np.asarray(o)
+    h = _h_per_sample(o.shape[-1], zero_padding, lamb, d, px, o.shape[0])
+    return propagate_h(o, h, zero_padding, adjoint)
+
+
+def asm_c64(o, lamb, d, px, zero_padding=False, adjoint=False) -> np.ndarray:
+    """The same operator as a plain complex64 pipeline: single-precision FFTs, H rounded to complex64.
+
+    A correct single-precision implementation; its distance from the float64 result calibrates the bounds of the
+    GPU parity tests (about 2-4e-7 rel-L2 on white fields).
+    """
+    o = np.asarray(o)
+    h = _h_per_sample(o.shape[-1], zero_padding, lamb, d, px, o.shape[0])
+    return propagate_h(o.astype(np.complex64), h, zero_padding, adjoint, dtype=np.complex64)
+
+
+def output_stage(u: np.ndarray, out_mode: int, out_scale: float = 1.0) -> list:
+    """What asm_b200_forward writes for ``out_mode`` (out0, then out1), computed in the precision of ``u``."""
+    real = np.float32 if u.dtype == np.complex64 else np.float64
+    s = real(out_scale)
+    if out_mode == OUT_COMPLEX:
+        return [u]
+    if out_mode == OUT_INTENSITY:
+        return [np.abs(u) ** 2, u]
+    if out_mode == OUT_ABS_ANGLE:
+        return [np.abs(u), np.angle(u)]
+    if out_mode == OUT_REIM_CAT:
+        return [np.concatenate([u.real * s, u.imag * s], axis=1)]
+    if out_mode == OUT_ABSANG_CAT:
+        su = u * s
+        return [np.concatenate([np.abs(su), np.angle(su)], axis=1)]
+    raise ValueError(f"out_mode {out_mode} is not a forward output")
+
+
+def grad_ap(go: np.ndarray, amplitude, phase, in_scale: float) -> list:
+    """OUT_GRAD_AP of the adjoint: [Re(conj(e) go), in_scale a Im(conj(e) go)], e = exp(i fl32(phase in_scale))."""
+    e = np.exp(1j * scaled_phase(phase, in_scale)).astype(go.dtype)
+    t = np.conj(e) * go
+    real = t.real.dtype.type
+    return [t.real, real(in_scale) * np.asarray(amplitude).astype(real) * t.imag]
+
+
+def asm_dudz(o, lamb, d, px, zero_padding=False):
+    """(U, dU/dz) from one spectrum: U = crop(ifft2(H F)), dU/dz = crop(ifft2(i K kz H F)), F = fft2(pad(o)), K =
+    ``grad_constant(d)``.  complex128 [B,C,N,N] each."""
+    o = np.asarray(o)
+    b, _, n, _ = o.shape
+    m = 2 * n if zero_padding else n
+    p = (m - n) // 2
+    idx = np.clip(np.arange(m) - p, 0, n - 1)
+    fft2, ifft2 = _fft_pair()
+    d = _as_b(d, b)
+    hf = transfer_function(m, n, lamb, px, d)[:, None] * fft2(o.astype(np.complex128)[:, :, idx][:, :, :, idx])
+    u = ifft2(hf)[:, :, p:p + n, p:p + n]
+    du = ifft2((1j * grad_constant(d) * kz_unshifted(m, n, lamb, px)) * hf)[:, :, p:p + n, p:p + n]
+    return u, du
+
+
+def grad_z_sum(g, u, du, lamb, d, kshift=0.0):
+    """grad_z[b] = Re sum_{c,y,x} conj(g) dU/dz and its rounding scale S_b = sum |Re(conj(g) dU/dz)|, float64 [B] each.
+
+    With kshift = 1 the derivative is taken with kz - 1/lamb in place of kz, i.e. dU/dz - i K U / lamb: the form the
+    library evaluates for the intensity cotangent (asm_b200_grad_z).  It gives the same gradient when g = 2 w U.
+    """
+    if kshift:
+        du = du - (1j * grad_constant(d) * kshift / lamb) * u
+    t = np.real(np.conj(np.asarray(g).astype(np.complex128)) * du)
+    return t.sum(axis=(1, 2, 3)), np.abs(t).sum(axis=(1, 2, 3))
+
+
+def asm_grad_z(o, g, lamb, d, px, zero_padding=False, kshift=0.0):
+    """``grad_z_sum`` of U = asm(o) (see there): returns (grad [B], S [B])."""
+    u, du = asm_dudz(o, lamb, d, px, zero_padding)
+    return grad_z_sum(g, u, du, lamb, np.asarray(_as_b(d, np.asarray(o).shape[0])), kshift)
+
+
 def rel_l2(a, b) -> float:
     a = np.asarray(a)
     b = np.asarray(b)
