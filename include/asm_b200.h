@@ -119,7 +119,9 @@ int asm_b200_grad_z(const void* in0, const void* in1, const void* z, int z_dtype
  * image) that Holo_Generator.forward(..., return_field=True, unwrap=True) calls (utils/Forward_model.py:31-32,
  * test_field_retrieval_mnist.py:126).  Same algorithm as scikit-image's 2-D unwrap_phase (Herraez et al. 2002: sort edges by
  * reliability, merge pixel groups along them); ties are broken by edge index instead of skimage's RNG, so results agree
- * wherever the wrapped phase has no residues.  out may alias phase.  Workspace: asm_b200_unwrap_workspace_bytes.
+ * wherever the wrapped phase has no residues.  out = fl32(phase + 2 pi k) per pixel, k an integer and the sum in double.
+ * out may alias phase.  Shapes: H, W >= 3, H W <= 2^28 and B (2 H W - H - W) <= INT_MAX (edges of the batch); any other
+ * shape returns ASM_B200_E_SHAPE, and asm_b200_unwrap_workspace_bytes returns 0 for exactly those shapes.
  */
 size_t asm_b200_unwrap_workspace_bytes(int B, int H, int W);
 int asm_b200_unwrap(const float* phase, float* out, int B, int H, int W,

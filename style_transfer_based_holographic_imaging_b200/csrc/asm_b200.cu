@@ -1800,8 +1800,7 @@ extern "C" int asm_b200_unwrap(const float* phase, float* out, int B, int H, int
     if (!phase || !out) return ASM_B200_E_NULL;
     UnwrapLayout L;
     if (!unwrap_layout(B, H, W, &L)) return ASM_B200_E_SHAPE;
-    const long long E = (long long)B * ((long long)H * (W - 1) + (long long)(H - 1) * W);
-    if (E > 0x7fffffffll) return ASM_B200_E_SHAPE;
+    const long long E = (long long)B * ((long long)H * (W - 1) + (long long)(H - 1) * W);   // <= INT_MAX (unwrap_layout)
     if (!workspace || ((uintptr_t)workspace & 255) || workspace_bytes < L.total) return ASM_B200_E_WORKSPACE;
     int rc = check_device();
     if (rc) return rc;

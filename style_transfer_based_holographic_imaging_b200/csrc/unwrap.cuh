@@ -14,7 +14,7 @@
 //   4. edges are visited in that order; two pixels of different groups merge their groups, the group that joins is shifted
 //      by the multiple of 2 pi that makes the edge consistent: a single pixel joins its neighbour's group, otherwise the
 //      group with fewer pixels joins the larger one (ties: the first pixel's group joins);
-//   5. unwrapped = wrapped + 2 pi * increment.
+//   5. unwrapped = fl32(wrapped + 2 pi * increment), the sum in double.
 // Step 4 is sequential per image (a weighted union-find with per-node offsets, one thread per image, images in parallel);
 // everything else is data parallel.
 #pragma once
@@ -163,21 +163,26 @@ __global__ void k_unwrap_merge_smem(const float* __restrict__ ph_g, const int* _
     }
 }
 
-__global__ void k_unwrap_apply(const float* __restrict__ ph, float* __restrict__ out, const int* __restrict__ parent,
+// unwrapped = fl32(ph + 2 pi k) with the sum in double: the value the reference's float64 unwrap gives after its callers'
+// .float().  (ph and out are not __restrict__: out may alias ph.)
+__global__ void k_unwrap_apply(const float* ph, float* out, const int* __restrict__ parent,
                                const int* __restrict__ off, const int* __restrict__ base, int B, int P) {
     const size_t n = (size_t)B * P;
     for (size_t idx = blockIdx.x * (size_t)blockDim.x + threadIdx.x; idx < n; idx += (size_t)gridDim.x * blockDim.x) {
         const size_t img = idx / P * P;
         int x = (int)(idx - img), acc = 0;
         while (parent[img + x] != x) { acc += off[img + x]; x = parent[img + x]; }
-        out[idx] = ph[idx] + 6.28318530717958647692f * (float)(acc + base[img + x]);
+        out[idx] = __double2float_rn(__dadd_rn((double)ph[idx], __dmul_rn(6.283185307179586476925, (double)(acc + base[img + x]))));
     }
 }
 
 struct UnwrapLayout { size_t rel, key_in, key_out, id_in, id_out, seg, parent, off, size, base, cub, cub_bytes, total; };
 
+// false for every shape asm_b200_unwrap rejects, so that asm_b200_unwrap_workspace_bytes reports 0 for exactly those:
+// H, W >= 3, H W <= 2^28, and B E <= INT_MAX (E edges per image; cub's item count and the segment offsets are ints).
 static bool unwrap_layout(int B, int H, int W, UnwrapLayout* L) {
     if (B <= 0 || H < 3 || W < 3 || (long long)H * W > (1ll << 28)) return false;
+    if ((long long)B * ((long long)H * (W - 1) + (long long)(H - 1) * W) > 0x7fffffffll) return false;
     const size_t P = (size_t)B * H * W, E = (size_t)B * ((size_t)H * (W - 1) + (size_t)(H - 1) * W);
     size_t o = 0;
     auto take = [&](size_t bytes) { const size_t at = o; o += (bytes + 255) / 256 * 256; return at; };

@@ -341,12 +341,13 @@ def unwrap_phase(x: torch.Tensor) -> torch.Tensor:
     else:
         raise RuntimeError("unwrap_phase expects [B, 1, H, W], [B, H, W] or [H, W]")
     lib = L.load()
+    need = lib.asm_b200_unwrap_workspace_bytes(b, h, w)
+    if need == 0:
+        raise RuntimeError(f"unwrap_phase: unsupported shape {tuple(x.shape)} "
+                           "(H, W >= 3, H W <= 2^28, B (2 H W - H - W) <= 2^31 - 1)")
     ph = x.detach().to(torch.float32).contiguous()
     out = torch.empty((b, 1, h, w), dtype=torch.float32, device=x.device)
     with torch.cuda.device(x.device):
-        need = lib.asm_b200_unwrap_workspace_bytes(b, h, w)
-        if need == 0:
-            raise RuntimeError(f"unwrap_phase: unsupported shape {tuple(x.shape)} (H, W >= 3)")
         ws = torch.empty(need, dtype=torch.uint8, device=x.device)
         L.check(lib.asm_b200_unwrap(ph.data_ptr(), out.data_ptr(), b, h, w, ws.data_ptr(), need,
                                     torch.cuda.current_stream().cuda_stream))
