@@ -151,6 +151,44 @@ int asm_b200_focal_stack(const void* in0, const void* in1, const void* z, int z_
                          double lambda, double px, float in_scale,
                          void* workspace, size_t workspace_bytes, void* stream);
 
+/*
+ * Band-limited angular spectrum (Matsushima & Shimobaba, Opt. Express 17, 19662, 2009).  Past a distance that depends
+ * on the grid, the phase chirp of H is undersampled on the FFT grid and its bins alias (ghost fringes wrapped around the
+ * window).  The _bl entry points take the arguments of their counterparts above plus `band_limit`:
+ *   band_limit = 0: exactly the counterpart (the counterparts are these calls with band_limit = 0: same launches, same bits);
+ *   band_limit = 1: for every plane, with z its distance as a double (an fp32 z converts exactly) and S = M px in double,
+ *       lim(z) = floor( S / (lambda sqrt(1 + q q)) ),  q = 2 z / S       (double, this operation order, no contraction;
+ *                                                                          clamped to M before the conversion to int)
+ *     bin (u, v) is kept iff |k(u)| <= lim and |k(v)| <= lim, k(u) = u < M/2 ? u : u - M (the signed frequency index):
+ *     i.e. |f_x|, |f_y| <= 1 / (lambda sqrt(1 + (2 z df)^2)), df = 1 / (M px).  Kept bins get H unchanged (including the
+ *     evanescent clamp H = 1); the others get H = 0.  Forward: H mask; adjoint: conj(H) mask; distance derivative:
+ *     i K kz H mask.  The mask is piecewise constant in z and is treated as a constant: the loss jumps where lim(z)
+ *     changes, and grad_z does not see those jumps.
+ *   any other value: ASM_B200_E_MODE.
+ * Opt-in only: where lim >= M/2 (short distances, fine grids) the result equals the plain call bit for bit, and at short
+ * distances the plain spectrum is the more accurate one.
+ */
+int asm_b200_forward_bl(const void* in0, const void* in1, const void* z, int z_dtype,
+                        void* out0, void* out1,
+                        int B, int C, int N, int pad, int in_mode, int out_mode,
+                        double lambda, double px, float in_scale, float out_scale,
+                        void* workspace, size_t workspace_bytes, void* stream, int band_limit);
+int asm_b200_adjoint_bl(const void* in0, const void* in1, const void* z, int z_dtype,
+                        const void* aux0, const void* aux1, void* out0, void* out1,
+                        int B, int C, int N, int pad, int in_mode, int out_mode,
+                        double lambda, double px, float in_scale,
+                        void* workspace, size_t workspace_bytes, void* stream, int band_limit);
+int asm_b200_grad_z_bl(const void* in0, const void* in1, const void* z, int z_dtype,
+                       const void* cot0, const void* cot1, int cot_mode, double* grad_z,
+                       int B, int C, int N, int pad, int in_mode,
+                       double lambda, double px, float in_scale,
+                       void* workspace, size_t workspace_bytes, void* stream, int band_limit);
+int asm_b200_focal_stack_bl(const void* in0, const void* in1, const void* z, int z_dtype, int K,
+                            void* out0, void* out1, double* moments,
+                            int B, int N, int pad, int in_mode, int out_mode,
+                            double lambda, double px, float in_scale,
+                            void* workspace, size_t workspace_bytes, void* stream, int band_limit);
+
 /* Number of CUDA kernels this library has launched in this process so far (all threads, all devices).
  * Instrumentation for bench.py (`gpu_launches`); not part of the reference's interface. */
 unsigned long long asm_b200_launch_count(void);
@@ -164,7 +202,7 @@ void asm_b200_profile(int enable, double* ms3);
 /* error codes (negative return values) */
 #define ASM_B200_E_NULL        (-1) /* a required pointer is NULL                      */
 #define ASM_B200_E_SHAPE       (-2) /* unsupported N (see Conventions) / B,C <= 0        */
-#define ASM_B200_E_MODE        (-3) /* unknown or inconsistent in_mode / out_mode      */
+#define ASM_B200_E_MODE        (-3) /* unknown or inconsistent in_mode / out_mode / band_limit */
 #define ASM_B200_E_WORKSPACE   (-4) /* workspace too small or misaligned (256 B)       */
 #define ASM_B200_E_OPTICS      (-5) /* lambda or px not finite and positive            */
 #define ASM_B200_E_DRIVER      (-6) /* cuTensorMapEncodeTiled unavailable / failed     */

@@ -6,6 +6,8 @@ Constructor and ``forward`` signatures are those of the reference (``utils/Forwa
 
 Deviations (SURVEY.md section 8b): CUDA tensors only; ``complex_number=True`` returns complex64 and
 ``Back_prop`` returns float32 (reference: complex128 / float64) unless ``ref_dtype=True`` is set on the module.
+``band_limit=True`` on either constructor (opt-in, not in the reference) propagates with the band-limited angular
+spectrum (see ``ASM``); the ``forward`` signatures stay the reference's.
 """
 from __future__ import annotations
 
@@ -43,7 +45,7 @@ def _broadcast_amp_phase(amplitude, phase):
 class Holo_Generator(nn.Module):
     """Free-space forward model: complex object field -> hologram at distance d (utils/Forward_model.py:6-39)."""
 
-    def __init__(self, args, ref_dtype: bool = False):
+    def __init__(self, args, ref_dtype: bool = False, band_limit: bool = False):
         super().__init__()
         self.wavelength = args.wavelength
         self.pixel_size = args.pixel_size
@@ -51,27 +53,28 @@ class Holo_Generator(nn.Module):
         self.distance_normalize_constant = args.distance_normalize_constant
         self.phase_normalize = args.phase_normalize
         self.ref_dtype = ref_dtype
+        self.band_limit = bool(band_limit)
 
     def forward(self, amplitude, phase, d, return_field=False, complex_number=False, unwrap=False):
         # normalised mm -> metres with the reference's fp32 rounding sequence (utils/Forward_model.py:18)
         d = ((d + self.distance_normalize_constant) * self.distance_normalize) * 1e-3
-        lamb, px, pn = self.wavelength, self.pixel_size, self.phase_normalize
+        lamb, px, pn, bl = self.wavelength, self.pixel_size, self.phase_normalize, self.band_limit
         amplitude, phase = _broadcast_amp_phase(amplitude, phase)
         needs_graph = torch.is_grad_enabled() and any(
             isinstance(t, torch.Tensor) and t.requires_grad for t in (amplitude, phase, d))
         if return_field:
             if needs_graph:
-                U = F_.HoloField.apply(amplitude, phase, d, lamb, px, pn, True)
+                U = F_.HoloField.apply(amplitude, phase, d, lamb, px, pn, True, bl)
                 amp_prop, ph_prop = torch.abs(U), torch.angle(U)
             else:
-                amp_prop, ph_prop = F_.holo_abs_angle(amplitude, phase, d, lamb, px, pn, True)
+                amp_prop, ph_prop = F_.holo_abs_angle(amplitude, phase, d, lamb, px, pn, True, bl)
             if unwrap:
                 ph_prop = F_.unwrap_phase(ph_prop)        # (the keyword argument shadows the module-level unwrap)
             return amp_prop, ph_prop
         if complex_number:
-            U = F_.HoloField.apply(amplitude, phase, d, lamb, px, pn, True)
+            U = F_.HoloField.apply(amplitude, phase, d, lamb, px, pn, True, bl)
             return U.to(torch.complex128) if self.ref_dtype else U
-        return F_.HoloIntensity.apply(amplitude, phase, d, lamb, px, pn, True)
+        return F_.HoloIntensity.apply(amplitude, phase, d, lamb, px, pn, True, bl)
 
     @torch.no_grad()
     def forward_pair(self, amplitude, phase_a, phase_b, d_a, d_b):
@@ -88,15 +91,17 @@ class Holo_Generator(nn.Module):
         amp_b, phase_b = _broadcast_amp_phase(amplitude, phase_b)
         if amp_a.numel() == 1 or amp_a.data_ptr() == amp_b.data_ptr():
             return F_.holo_intensity_pair(amp_a, phase_a, phase_b, d_a, d_b, self.wavelength, self.pixel_size,
-                                          self.phase_normalize, True)
-        return (F_.HoloIntensity.apply(amp_a, phase_a, d_a, self.wavelength, self.pixel_size, self.phase_normalize, True),
-                F_.HoloIntensity.apply(amp_b, phase_b, d_b, self.wavelength, self.pixel_size, self.phase_normalize, True))
+                                          self.phase_normalize, True, self.band_limit)
+        return (F_.HoloIntensity.apply(amp_a, phase_a, d_a, self.wavelength, self.pixel_size, self.phase_normalize, True,
+                                       self.band_limit),
+                F_.HoloIntensity.apply(amp_b, phase_b, d_b, self.wavelength, self.pixel_size, self.phase_normalize, True,
+                                       self.band_limit))
 
 
 class Back_prop(nn.Module):
     """Back-propagated hologram as network input (utils/Forward_model.py:42-65)."""
 
-    def __init__(self, args, ref_dtype: bool = False):
+    def __init__(self, args, ref_dtype: bool = False, band_limit: bool = False):
         super().__init__()
         self.amplitude_normalize = args.amplitude_normalize
         self.wavelength = args.wavelength
@@ -105,6 +110,7 @@ class Back_prop(nn.Module):
         self.distance_normalize_constant = args.distance_normalize_constant
         self.input_type = args.Holo_G_input
         self.ref_dtype = ref_dtype
+        self.band_limit = bool(band_limit)
 
     def forward(self, holo, d):
         d = ((d + self.distance_normalize_constant) * self.distance_normalize) * 0.001
@@ -112,9 +118,10 @@ class Back_prop(nn.Module):
         needs_graph = torch.is_grad_enabled() and any(
             isinstance(t, torch.Tensor) and t.requires_grad for t in (holo, d))
         if needs_graph:
-            U = ASM(torch.sqrt(holo), self.wavelength, d, self.pixel_size) * self.amplitude_normalize
+            U = ASM(torch.sqrt(holo), self.wavelength, d, self.pixel_size, band_limit=self.band_limit) * self.amplitude_normalize
             r, i = (torch.abs(U), torch.angle(U)) if amp_pha else (torch.real(U), torch.imag(U))
             out = torch.cat([r, i], dim=1)
         else:
-            out = F_.back_prop_fused(holo, d, self.wavelength, self.pixel_size, self.amplitude_normalize, amp_pha)
+            out = F_.back_prop_fused(holo, d, self.wavelength, self.pixel_size, self.amplitude_normalize, amp_pha,
+                                     self.band_limit)
         return out.to(torch.float64) if self.ref_dtype else out

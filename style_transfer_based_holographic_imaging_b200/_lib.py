@@ -17,7 +17,8 @@ ABI_VERSION = 1
 SYMBOLS = ["asm_b200_abi_version", "asm_b200_strerror", "asm_b200_workspace_bytes", "asm_b200_forward",
            "asm_b200_adjoint", "asm_b200_grad_z", "asm_b200_launch_count", "asm_b200_profile",
            "asm_b200_unwrap_workspace_bytes", "asm_b200_unwrap", "asm_b200_focal_stack_workspace_bytes",
-           "asm_b200_focal_stack"]
+           "asm_b200_focal_stack", "asm_b200_forward_bl", "asm_b200_adjoint_bl", "asm_b200_grad_z_bl",
+           "asm_b200_focal_stack_bl"]
 
 _lib = None
 
@@ -60,6 +61,14 @@ def load() -> ctypes.CDLL:
     lib.asm_b200_focal_stack_workspace_bytes.argtypes = [ci, ci, ci, ci]
     lib.asm_b200_focal_stack.restype = ci
     lib.asm_b200_focal_stack.argtypes = [vp, vp, vp, ci, ci, vp, vp, vp, ci, ci, ci, ci, ci, cd, cd, cf, vp, sz, vp]
+    # the band-limited entry points: the arguments of their counterparts plus a trailing int band_limit (an older build
+    # loaded through ASM_B200_LIB for an A/B comparison has none; band-limited calls then raise)
+    for name in ("asm_b200_forward", "asm_b200_adjoint", "asm_b200_grad_z", "asm_b200_focal_stack"):
+        if not hasattr(lib, name + "_bl"):
+            continue
+        fn = getattr(lib, name + "_bl")
+        fn.restype = ci
+        fn.argtypes = getattr(lib, name).argtypes + [ci]
     if lib.asm_b200_abi_version() != ABI_VERSION:
         raise AsmB200Error("libasm_b200.so ABI version mismatch; rebuild it")
     _lib = lib

@@ -37,9 +37,11 @@ struct Params {
     double inv_lambda;                    // 1 / lambda
     double lambda;
     double kshift;                        // H_DERIV: the filter is i (kz - kshift / lambda) H (see asm_b200_grad_z)
+    double S;                             // M px: the window of the FFT grid (band limit)
     float in_scale, out_scale, inv_m2;
     int planes, C, N, M, P;               // planes = B*C
     int in_mode, out_mode, aux_mode, h_mode, adj, z_f64;
+    int band_limit;                       // 1: zero the bins outside the band limit of each plane's z (band_limit_of)
     // focal stack (asm_b200_focal_stack): planes are (sample, distance) pairs q = b kst + k.  The column pass reads the
     // spectrum of sample q / kst from src (slot q / kst - s0) and writes plane q to ws; kst = 0 outside a stack.
     const float2* src;
@@ -95,6 +97,18 @@ __device__ __forceinline__ double phase_constant_of(const Params& p, int b) {
     if (p.z_f64) cph = 6.283185307179586 * __ldg((const double*)p.z + b);
     else cph = (double)__fmul_rn(6.2831854820251465f, __ldg((const float*)p.z + b));
     return p.h_mode == H_CONJ ? -cph : cph;
+}
+
+// Band limit of a sample (Matsushima & Shimobaba, Opt. Express 17, 19662, 2009): bin (u, v) is kept iff |k(u)| <= lim
+// and |k(v)| <= lim, lim = floor(S / (lambda sqrt(1 + q^2))), q = 2 z / S, S = M px, in double in exactly this order
+// (no contraction), clamped to M before the conversion (S / lambda may exceed INT_MAX; a NaN z keeps every bin).
+// Without the band limit every bin is kept (lim = M > M / 2).  The only statement of the rule on the device.
+__device__ __forceinline__ int band_limit_of(const Params& p, int b) {
+    if (!p.band_limit) return p.M;
+    const double z = p.z_f64 ? __ldg((const double*)p.z + b) : (double)__ldg((const float*)p.z + b);
+    const double q = __ddiv_rn(__dmul_rn(2.0, z), p.S);
+    const double t = __ddiv_rn(p.S, __dmul_rn(p.lambda, __dsqrt_rn(__dadd_rn(1.0, __dmul_rn(q, q)))));
+    return (int)fmin(floor(t), (double)p.M);
 }
 
 // ---------------------------------------------------------------------------------------------------
@@ -480,7 +494,8 @@ __host__ __device__ constexpr bool kz_in_smem(int n) { return n <= 10 || (n == 1
 #endif
 __host__ __device__ constexpr int cols_min_blocks(int n) { return n <= 8 ? 4 : n <= 10 ? (1024 / (cols_per_slab(n) * (1 << n) / 16)) : n == 11 ? ASM_MB11 : (ASM_CC12 <= 2 ? 2 : 1); }
 
-template <int n>
+// BL: band-limited calls (p.band_limit; a template parameter so that the plain instantiations stay the code they were)
+template <int n, bool BL = false>
 __global__ void __launch_bounds__(cols_per_slab(n) * (1 << n) / 16, cols_min_blocks(n))
 k_cols(const Params p, const __grid_constant__ CUtensorMap tmap, const __grid_constant__ CUtensorMap tmap_src,
        const __grid_constant__ CUtensorMap tmap_kz, int plane0) {
@@ -526,6 +541,12 @@ k_cols(const Params p, const __grid_constant__ CUtensorMap tmap, const __grid_co
     if (p.z_f64) cph = 6.283185307179586 * __ldg((const double*)p.z + b);
     else cph = (double)__fmul_rn(6.2831854820251465f, __ldg((const float*)p.z + b));
     if (p.h_mode == H_CONJ) cph = -cph;
+    // band limit: this column's |k(v)| is within it -> rows |k(u)| <= lim_u are kept; otherwise none (lim_u = -1)
+    int lim_u = L;
+    if constexpr (BL) {
+        const int vpos = freq_of_pos(n, slab_i * CC + c), lim = band_limit_of(p, b);
+        lim_u = (vpos <= L / 2 ? vpos : L - vpos) <= lim ? lim : -1;
+    }
 
     mbar_wait(bar, 0);
     if (p.P > 0) {
@@ -560,9 +581,9 @@ k_cols(const Params p, const __grid_constant__ CUtensorMap tmap, const __grid_co
 #pragma unroll
         for (int i = 0; i < 16; ++i) {
             const int u = Q + TPL * i;
+            const int ru = u <= L / 2 ? u : L - u;                   // |k(u)|
             double tt, kzl = 0.0;
             if constexpr (KZTAB || KZGLOB) {
-                const int ru = u <= L / 2 ? u : L - u;
                 const double kap = KZTAB ? kz_s[ru * CC + c] : __ldg(p.kzt + (size_t)ru * L + slab_i * CC + c);
                 tt = kap * cph;
                 if (p.h_mode == H_DERIV) kzl = kap * (6.283185307179586 * p.lambda);
@@ -576,8 +597,9 @@ k_cols(const Params p, const __grid_constant__ CUtensorMap tmap, const __grid_co
             const double rr = tt - __dadd_rn(__dadd_rn(tt, MAGIC), -MAGIC);
             float sn, cn;
             __sincosf((float)rr * 6.283185307179586f, &sn, &cn);
-            if (p.h_mode == H_DERIV) v[i] = cmul_scaled(v[i], -sn, cn, (float)(kzl - p.kshift) * p.inv_m2);
-            else v[i] = cmul_scaled(v[i], cn, sn, p.inv_m2);
+            const float sc = (!BL || ru <= lim_u) ? p.inv_m2 : 0.f;  // H = 0 outside the band limit
+            if (p.h_mode == H_DERIV) v[i] = cmul_scaled(v[i], -sn, cn, (float)(kzl - p.kshift) * sc);
+            else v[i] = cmul_scaled(v[i], cn, sn, sc);
         }
     }
 
@@ -833,6 +855,7 @@ static cudaError_t set_attrs(size_t smem_fwd, size_t smem_inv, size_t smem_cols)
     if ((e = set_smem(k_rows_inv<n>, smem_inv)) != cudaSuccess) return e;
     if ((e = set_smem(k_rows_inv<n, true>, smem_inv)) != cudaSuccess) return e;
     if ((e = set_smem(k_cols<n>, smem_cols)) != cudaSuccess) return e;
+    if ((e = set_smem(k_cols<n, true>, smem_cols)) != cudaSuccess) return e;
     attrs_mark(done, dev);
     return cudaSuccess;
 }
@@ -877,10 +900,11 @@ static CallKey make_key(const Params& p, const Geometry& g, int kind, const Stac
     memset(&k, 0, sizeof(k));
     key_add(k, p.in0); key_add(k, p.in1); key_add(k, p.aux0); key_add(k, p.aux1); key_add(k, p.out0); key_add(k, p.out1);
     key_add(k, p.z); key_add(k, p.ws); key_add(k, p.tw); key_add(k, p.tw32); key_add(k, p.kzt);
-    key_add(k, p.s2); key_add(k, p.inv_lambda); key_add(k, p.lambda); key_add(k, p.kshift);
+    key_add(k, p.s2); key_add(k, p.inv_lambda); key_add(k, p.lambda); key_add(k, p.kshift); key_add(k, p.S);
     key_add(k, p.in_scale); key_add(k, p.out_scale); key_add(k, p.inv_m2);
     key_add(k, p.planes); key_add(k, p.C); key_add(k, p.N); key_add(k, p.M); key_add(k, p.P);
     key_add(k, p.in_mode); key_add(k, p.out_mode); key_add(k, p.aux_mode); key_add(k, p.h_mode); key_add(k, p.adj); key_add(k, p.z_f64);
+    key_add(k, p.band_limit);
     key_add(k, g.n); key_add(k, g.chunk); key_add(k, g.lanes); key_add(k, g.cc); key_add(k, kind);
     const int stack = sp != nullptr;
     key_add(k, stack);
@@ -1079,6 +1103,7 @@ static int launch_n(const Params& p0, const Geometry& g, cudaStream_t st, const 
         const int ntiles = (nlines + LPC - 1) / LPC;
         const int grid_rows = ntiles < row_ctas_max ? ntiles : row_ctas_max;
         if (k == 0) k_rows_fwd<n><<<grid_rows, ROW_THREADS, smem_fwd, s>>>(p, plane0, nlines, ntiles);
+        else if (k == 1 && p.band_limit) k_cols<n, true><<<nimg * (L / CC), CC * TPL, smem_cols, s>>>(p, tmap_t[lane], tmap[lane], tmap_kz, plane0);
         else if (k == 1) k_cols<n><<<nimg * (L / CC), CC * TPL, smem_cols, s>>>(p, tmap_t[lane], tmap[lane], tmap_kz, plane0);
         else if (p.part) k_rows_inv<n, true><<<grid_rows, ROW_THREADS, smem_inv, s>>>(p, plane0, nlines, ntiles);
         else k_rows_inv<n><<<grid_rows, ROW_THREADS, smem_inv, s>>>(p, plane0, nlines, ntiles);
@@ -1321,6 +1346,7 @@ static int launch_32t(const Params& p0, const Geometry& g, cudaStream_t st, cons
             K32T_SET((k32t_rows_inv<1, false>), K32T_INV_SMEM) K32T_SET((k32t_rows_inv<1, true>), K32T_INV_SMEM)
             K32T_SET((k32t_rows_inv<2, false>), K32T_INV_SMEM) K32T_SET((k32t_rows_inv<2, true>), K32T_INV_SMEM)
             K32T_SET((k32t_lines<false>), K32T_LINES_SMEM) K32T_SET((k32t_lines<true>), K32T_LINES_SMEM)
+            K32T_SET((k32t_lines<false, true>), K32T_LINES_SMEM) K32T_SET((k32t_lines<true, true>), K32T_LINES_SMEM)
 #undef K32T_SET
             attrs_mark(done, dev);
         }
@@ -1364,8 +1390,10 @@ static int launch_32t(const Params& p0, const Geometry& g, cudaStream_t st, cons
             const int nlines = nimg * L;
             const int want = (nlines + K32T_LINE_WARPS - 1) / K32T_LINE_WARPS, cap = K32T_LINE_CTAS * sm_count();
             const int grid = want < cap ? want : cap;
-            if (padded) k32t_lines<true><<<grid, 32 * K32T_LINE_WARPS, K32T_LINES_SMEM, s>>>(p, plane0, nlines);
-            else k32t_lines<false><<<grid, 32 * K32T_LINE_WARPS, K32T_LINES_SMEM, s>>>(p, plane0, nlines);
+#define K32T_LINES(PAD, BL) k32t_lines<PAD, BL><<<grid, 32 * K32T_LINE_WARPS, K32T_LINES_SMEM, s>>>(p, plane0, nlines);
+            if (p.band_limit) { if (padded) K32T_LINES(true, true) else K32T_LINES(false, true) }
+            else { if (padded) K32T_LINES(true, false) else K32T_LINES(false, false) }
+#undef K32T_LINES
         } else {
             const int out = !inv_bulk ? 2 : p.out_mode == ASM_B200_OUT_INTENSITY ? 1 : 0;
             const int grid_inv = ngroups / 2 < cap_rows ? ngroups / 2 : cap_rows;   // pairs of groups
@@ -1412,6 +1440,10 @@ static int launch_64(const Params& p0, const Geometry& g, cudaStream_t st, const
             if ((e = set_smem(k64_cols<true, false>, K64_COLS_SMEM)) != cudaSuccess) return (int)e;
             if ((e = set_smem(k64_cols<false, true>, K64_COLS_SMEM)) != cudaSuccess) return (int)e;
             if ((e = set_smem(k64_cols<true, true>, K64_COLS_SMEM)) != cudaSuccess) return (int)e;
+            if ((e = set_smem(k64_cols<false, false, true>, K64_COLS_SMEM)) != cudaSuccess) return (int)e;
+            if ((e = set_smem(k64_cols<true, false, true>, K64_COLS_SMEM)) != cudaSuccess) return (int)e;
+            if ((e = set_smem(k64_cols<false, true, true>, K64_COLS_SMEM)) != cudaSuccess) return (int)e;
+            if ((e = set_smem(k64_cols<true, true, true>, K64_COLS_SMEM)) != cudaSuccess) return (int)e;
             attrs_mark(done, dev);
         }
     }
@@ -1424,7 +1456,7 @@ static int launch_64(const Params& p0, const Geometry& g, cudaStream_t st, const
                           q.out0 && !(sp && sp->mom);                // focal-stack moments: the generic row kernels
     const bool bulk = fwd_bulk && inv_bulk && knob_bulk() != 0;
 #ifdef ASM_B200_TUNING
-    if (bulk && knob_k64t() && q.N % 16 == 0) return launch_64t(p0, g, st);
+    if (bulk && knob_k64t() && q.N % 16 == 0) return q.band_limit ? ASM_B200_E_MODE : launch_64t(p0, g, st);   // k64t.cuh has no band limit
 #endif
     const bool padded = q.P > 0;
     auto setup = [&](cudaStream_t s) {
@@ -1441,13 +1473,14 @@ static int launch_64(const Params& p0, const Geometry& g, cudaStream_t st, const
         if (k == 1) {
             const int wk = nimg * (L / K64_CC), cap = 2 * sm_count();
             const int grid = wk < cap ? wk : cap;
+#define K64_COLS(PAD, PAIRS) { if (p.band_limit) k64_cols<PAD, PAIRS, true><<<grid, 64 * K64_CC, K64_COLS_SMEM, s>>>(p, plane0, nimg); \
+                                else k64_cols<PAD, PAIRS><<<grid, 64 * K64_CC, K64_COLS_SMEM, s>>>(p, plane0, nimg); }
             if (bulk) {   // the kappa table of the warp-pair row kernels holds (hi, lo) pairs
-                if (padded) k64_cols<true, true><<<grid, 64 * K64_CC, K64_COLS_SMEM, s>>>(p, plane0, nimg);
-                else k64_cols<false, true><<<grid, 64 * K64_CC, K64_COLS_SMEM, s>>>(p, plane0, nimg);
+                if (padded) K64_COLS(true, true) else K64_COLS(false, true)
             } else {
-                if (padded) k64_cols<true, false><<<grid, 64 * K64_CC, K64_COLS_SMEM, s>>>(p, plane0, nimg);
-                else k64_cols<false, false><<<grid, 64 * K64_CC, K64_COLS_SMEM, s>>>(p, plane0, nimg);
+                if (padded) K64_COLS(true, false) else K64_COLS(false, false)
             }
+#undef K64_COLS
             return;
         }
         if (!bulk) {
@@ -1606,6 +1639,7 @@ static int run(Params p, int B, int C, int N, int pad, double lambda, double px,
         p.planes = B * C; p.C = C; p.N = N; p.M = dg.M; p.P = dg.P;
         const double sd = lambda / ((double)dg.M * px);
         p.s2 = sd * sd; p.lambda = lambda; p.inv_lambda = 1.0 / lambda;
+        p.S = (double)dg.M * px;
         p.inv_m2 = 1.0f / ((float)dg.M * (float)dg.M);
         return launch_dft(p, dg, reinterpret_cast<unsigned char*>(workspace), reinterpret_cast<cudaStream_t>(stream));
     }
@@ -1619,8 +1653,13 @@ static int run(Params p, int B, int C, int N, int pad, double lambda, double px,
     p.s2 = s * s;
     p.lambda = lambda;
     p.inv_lambda = 1.0 / lambda;
+    p.S = (double)g.M * px;
     p.inv_m2 = 1.0f / ((float)g.M * (float)g.M);
     cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+#ifdef ASM_B200_TUNING
+    // the measured alternatives of tuning builds (resident.cuh, cluster256.cuh, k32_cols.cuh) have no band limit
+    if (p.band_limit && (g.resident || (g.n == 8 && knob_cluster256()) || (g.n == 10 && !knob_k32t()))) return ASM_B200_E_MODE;
+#endif
 #if defined(ASM_B200_TUNING) && !defined(ASM_B200_ONLY_1024)
     if (g.resident) {
         switch (g.n) {
@@ -1668,7 +1707,7 @@ extern "C" const char* asm_b200_strerror(int code) {
         case 0: return "ok";
         case ASM_B200_E_NULL: return "asm_b200: a required pointer is NULL";
         case ASM_B200_E_SHAPE: return "asm_b200: unsupported shape (square N: a power of two with 32 <= FFT size <= 4096, or any other even N with FFT size <= 2048; B, C > 0)";
-        case ASM_B200_E_MODE: return "asm_b200: unknown or inconsistent in_mode / out_mode";
+        case ASM_B200_E_MODE: return "asm_b200: unknown or inconsistent in_mode / out_mode, or band_limit not 0 or 1";
         case ASM_B200_E_WORKSPACE: return "asm_b200: workspace too small or not 256-byte aligned";
         case ASM_B200_E_OPTICS: return "asm_b200: wavelength and pixel size must be finite and positive";
         case ASM_B200_E_DRIVER: return "asm_b200: cuTensorMapEncodeTiled unavailable or failed";
@@ -1740,6 +1779,15 @@ static bool needs_in1(int in_mode) { return in_mode == ASM_B200_IN_AMP_PHASE || 
 extern "C" int asm_b200_forward(const void* in0, const void* in1, const void* z, int z_dtype, void* out0, void* out1,
                                 int B, int C, int N, int pad, int in_mode, int out_mode, double lambda, double px,
                                 float in_scale, float out_scale, void* workspace, size_t workspace_bytes, void* stream) {
+    return asm_b200_forward_bl(in0, in1, z, z_dtype, out0, out1, B, C, N, pad, in_mode, out_mode, lambda, px, in_scale,
+                               out_scale, workspace, workspace_bytes, stream, 0);
+}
+
+extern "C" int asm_b200_forward_bl(const void* in0, const void* in1, const void* z, int z_dtype, void* out0, void* out1,
+                                   int B, int C, int N, int pad, int in_mode, int out_mode, double lambda, double px,
+                                   float in_scale, float out_scale, void* workspace, size_t workspace_bytes, void* stream,
+                                   int band_limit) {
+    if (band_limit != 0 && band_limit != 1) return ASM_B200_E_MODE;
     if (in_mode < 0 || in_mode > ASM_B200_IN_CONST_AMP_PHASE || out_mode < 0 || out_mode > ASM_B200_OUT_ABSANG_CAT) return ASM_B200_E_MODE;
     if (z_dtype != ASM_B200_Z_F32 && z_dtype != ASM_B200_Z_F64) return ASM_B200_E_MODE;
     if ((out_mode == ASM_B200_OUT_REIM_CAT || out_mode == ASM_B200_OUT_ABSANG_CAT) && C != 1) return ASM_B200_E_MODE;
@@ -1747,7 +1795,7 @@ extern "C" int asm_b200_forward(const void* in0, const void* in1, const void* z,
     if (out_mode == ASM_B200_OUT_ABS_ANGLE && !out1) return ASM_B200_E_NULL;
     Params p{};
     p.in0 = in0; p.in1 = in1; p.out0 = out0; p.out1 = out1; p.z = z; p.z_f64 = z_dtype;
-    p.in_mode = in_mode; p.out_mode = out_mode; p.h_mode = H_FWD; p.adj = 0;
+    p.in_mode = in_mode; p.out_mode = out_mode; p.h_mode = H_FWD; p.adj = 0; p.band_limit = band_limit;
     p.in_scale = in_scale; p.out_scale = out_scale;
     return run(p, B, C, N, pad, lambda, px, workspace, workspace_bytes, stream);
 }
@@ -1756,6 +1804,15 @@ extern "C" int asm_b200_adjoint(const void* in0, const void* in1, const void* z,
                                 const void* aux1, void* out0, void* out1, int B, int C, int N, int pad, int in_mode,
                                 int out_mode, double lambda, double px, float in_scale, void* workspace,
                                 size_t workspace_bytes, void* stream) {
+    return asm_b200_adjoint_bl(in0, in1, z, z_dtype, aux0, aux1, out0, out1, B, C, N, pad, in_mode, out_mode, lambda, px,
+                               in_scale, workspace, workspace_bytes, stream, 0);
+}
+
+extern "C" int asm_b200_adjoint_bl(const void* in0, const void* in1, const void* z, int z_dtype, const void* aux0,
+                                   const void* aux1, void* out0, void* out1, int B, int C, int N, int pad, int in_mode,
+                                   int out_mode, double lambda, double px, float in_scale, void* workspace,
+                                   size_t workspace_bytes, void* stream, int band_limit) {
+    if (band_limit != 0 && band_limit != 1) return ASM_B200_E_MODE;
     if (in_mode != ASM_B200_IN_COMPLEX && in_mode != ASM_B200_IN_COT_FIELD) return ASM_B200_E_MODE;
     if (out_mode != ASM_B200_OUT_COMPLEX && out_mode != ASM_B200_OUT_GRAD_AP) return ASM_B200_E_MODE;
     if (z_dtype != ASM_B200_Z_F32 && z_dtype != ASM_B200_Z_F64) return ASM_B200_E_MODE;
@@ -1763,7 +1820,7 @@ extern "C" int asm_b200_adjoint(const void* in0, const void* in1, const void* z,
     if (out_mode == ASM_B200_OUT_GRAD_AP && (!aux0 || !aux1 || !out1)) return ASM_B200_E_NULL;
     Params p{};
     p.in0 = in0; p.in1 = in1; p.aux0 = aux0; p.aux1 = aux1; p.out0 = out0; p.out1 = out1; p.z = z; p.z_f64 = z_dtype;
-    p.in_mode = in_mode; p.out_mode = out_mode; p.h_mode = H_CONJ; p.adj = 1;
+    p.in_mode = in_mode; p.out_mode = out_mode; p.h_mode = H_CONJ; p.adj = 1; p.band_limit = band_limit;
     p.in_scale = in_scale; p.out_scale = 1.f;
     return run(p, B, C, N, pad, lambda, px, workspace, workspace_bytes, stream);
 }
@@ -1772,6 +1829,15 @@ extern "C" int asm_b200_grad_z(const void* in0, const void* in1, const void* z, 
                                const void* cot1, int cot_mode, double* grad_z, int B, int C, int N, int pad, int in_mode,
                                double lambda, double px, float in_scale, void* workspace, size_t workspace_bytes,
                                void* stream) {
+    return asm_b200_grad_z_bl(in0, in1, z, z_dtype, cot0, cot1, cot_mode, grad_z, B, C, N, pad, in_mode, lambda, px,
+                              in_scale, workspace, workspace_bytes, stream, 0);
+}
+
+extern "C" int asm_b200_grad_z_bl(const void* in0, const void* in1, const void* z, int z_dtype, const void* cot0,
+                                  const void* cot1, int cot_mode, double* grad_z, int B, int C, int N, int pad, int in_mode,
+                                  double lambda, double px, float in_scale, void* workspace, size_t workspace_bytes,
+                                  void* stream, int band_limit) {
+    if (band_limit != 0 && band_limit != 1) return ASM_B200_E_MODE;
     if (in_mode < 0 || in_mode > ASM_B200_IN_CONST_AMP_PHASE) return ASM_B200_E_MODE;
     if (cot_mode != ASM_B200_IN_COMPLEX && cot_mode != ASM_B200_IN_COT_FIELD) return ASM_B200_E_MODE;
     if (z_dtype != ASM_B200_Z_F32 && z_dtype != ASM_B200_Z_F64) return ASM_B200_E_MODE;
@@ -1782,7 +1848,7 @@ extern "C" int asm_b200_grad_z(const void* in0, const void* in1, const void* z, 
     if (e != cudaSuccess) return (int)e;
     Params p{};
     p.in0 = in0; p.in1 = in1; p.aux0 = cot0; p.aux1 = cot1; p.aux_mode = cot_mode; p.out0 = grad_z; p.z = z; p.z_f64 = z_dtype;
-    p.in_mode = in_mode; p.out_mode = OUT_DOT; p.h_mode = H_DERIV; p.adj = 0;
+    p.in_mode = in_mode; p.out_mode = OUT_DOT; p.h_mode = H_DERIV; p.adj = 0; p.band_limit = band_limit;
     // Intensity cotangent g = 2 w U: the constant part of kz contributes Re(conj(g) i k0 U) = 0 exactly, but in fp32 it
     // is a cancelling sum ~100x larger than the result.  Differentiate with kz - 1/lambda instead (same derivative).
     p.kshift = cot_mode == ASM_B200_IN_COT_FIELD ? 1.0 : 0.0;
@@ -1867,6 +1933,16 @@ extern "C" int asm_b200_focal_stack(const void* in0, const void* in1, const void
                                     int B, int N, int pad, int in_mode, int out_mode,
                                     double lambda, double px, float in_scale,
                                     void* workspace, size_t workspace_bytes, void* stream) {
+    return asm_b200_focal_stack_bl(in0, in1, z, z_dtype, K, out0, out1, moments, B, N, pad, in_mode, out_mode, lambda, px,
+                                   in_scale, workspace, workspace_bytes, stream, 0);
+}
+
+extern "C" int asm_b200_focal_stack_bl(const void* in0, const void* in1, const void* z, int z_dtype, int K,
+                                       void* out0, void* out1, double* moments,
+                                       int B, int N, int pad, int in_mode, int out_mode,
+                                       double lambda, double px, float in_scale,
+                                       void* workspace, size_t workspace_bytes, void* stream, int band_limit) {
+    if (band_limit != 0 && band_limit != 1) return ASM_B200_E_MODE;
     if (!out0 && !moments) return ASM_B200_E_NULL;
     if (in_mode < 0 || in_mode > ASM_B200_IN_CONST_AMP_PHASE || in_mode == ASM_B200_IN_COT_FIELD) return ASM_B200_E_MODE;
     if (out_mode != ASM_B200_OUT_COMPLEX && out_mode != ASM_B200_OUT_INTENSITY && out_mode != ASM_B200_OUT_ABS_ANGLE) return ASM_B200_E_MODE;
@@ -1883,7 +1959,7 @@ extern "C" int asm_b200_focal_stack(const void* in0, const void* in1, const void
     if (rc) return rc;
     Params p{};
     p.in0 = in0; p.in1 = in1; p.out0 = out0; p.out1 = out0 ? out1 : nullptr; p.z = z; p.z_f64 = z_dtype;
-    p.in_mode = in_mode; p.out_mode = out_mode; p.h_mode = H_FWD; p.adj = 0;
+    p.in_mode = in_mode; p.out_mode = out_mode; p.h_mode = H_FWD; p.adj = 0; p.band_limit = band_limit;
     p.in_scale = in_scale; p.out_scale = 1.f;
     p.C = 1; p.N = N; p.lambda = lambda; p.inv_lambda = 1.0 / lambda;
     cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
@@ -1896,6 +1972,7 @@ extern "C" int asm_b200_focal_stack(const void* in0, const void* in1, const void
         p.planes = B * K; p.M = dg.M; p.P = dg.P; p.kst = K;
         const double sd = lambda / ((double)dg.M * px);
         p.s2 = sd * sd;
+        p.S = (double)dg.M * px;
         p.inv_m2 = 1.0f / ((float)dg.M * (float)dg.M);
         p.part = moments ? reinterpret_cast<double*>(w + dft_workspace(dg)) : nullptr;
         return launch_dft(p, dg, w, st, moments);
@@ -1908,6 +1985,7 @@ extern "C" int asm_b200_focal_stack(const void* in0, const void* in1, const void
     p.ws = reinterpret_cast<float2*>(w + g.tw_bytes + g.kz_bytes);
     const double sd = lambda / ((double)g.M * px);
     p.s2 = sd * sd;
+    p.S = (double)g.M * px;
     p.inv_m2 = 1.0f / ((float)g.M * (float)g.M);
     switch (g.n) {
         case 5: return launch_n<5>(p, g, st, &sp);

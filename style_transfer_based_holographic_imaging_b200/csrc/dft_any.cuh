@@ -95,9 +95,11 @@ __device__ __forceinline__ float dft_emit_any(const Params& p, int plane, int y,
     }
 }
 
-// transfer function at bin (u, v), fp64 phase (same arithmetic as the kappa tables: ASM.py:16-29 on unshifted bins)
-__device__ __forceinline__ float2 dft_h(const Params& p, int u, int v, int M, double cph) {
+// transfer function at bin (u, v), fp64 phase (same arithmetic as the kappa tables: ASM.py:16-29 on unshifted bins);
+// 0 outside the band limit lim (band_limit_of)
+__device__ __forceinline__ float2 dft_h(const Params& p, int u, int v, int M, double cph, int lim) {
     const int ku = u < (M + 1) / 2 ? u : u - M, kv = v < (M + 1) / 2 ? v : v - M;
+    if (abs(ku) > lim || abs(kv) > lim) return make_float2(0.f, 0.f);
     const double arg = fma(-p.s2, (double)ku * ku + (double)kv * kv, 1.0);
     const double root = arg > 0.0 ? sqrt(arg) : 0.0;                 // kz lambda; evanescent -> 0 (H = 1)
     double t = root * p.inv_lambda * 0.15915494309189535 * cph;      // turns
@@ -162,14 +164,15 @@ __global__ void __launch_bounds__(256) k_dft_mm(const Params p, const float2* __
     float dot = 0.f;
     const int c = c0 + tx;
     double cph = 0.0;
-    if (KIND == 1) cph = phase_constant_of(p, plane / p.C);
+    int lim = 0;
+    if (KIND == 1) { cph = phase_constant_of(p, plane / p.C); lim = band_limit_of(p, plane / p.C); }
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
         const int r = r0 + ty + 8 * i;
         if (r >= R_ || c >= C_) continue;
         if (KIND == 0) T1[((size_t)img * N + r) * M + c] = acc[i];
         else if (KIND == 1) {
-            const float2 h = dft_h(p, c, r, M, cph);                 // column index = row-pass frequency u, row index = v
+            const float2 h = dft_h(p, c, r, M, cph, lim);                 // column index = row-pass frequency u, row index = v
             T2[((size_t)img * M + r) * M + c] = make_float2(acc[i].x * h.x - acc[i].y * h.y, acc[i].x * h.y + acc[i].y * h.x);
         } else if (KIND == 2) T3[((size_t)img * N + r) * M + c] = acc[i];
         else if (p.out0) dot += dft_emit_any(p, plane, r, c, acc[i]);

@@ -88,13 +88,15 @@ __device__ __forceinline__ int k32t_tile_idx(int u, int yy) { return u * 8 + (((
 // H(u, v = lane + 32 i) on the registers of one line.  c = (c_hi, c_lo): the sample's phase constant (ASM.py:29), negative
 // for the adjoint.  t = c kappa: p = hi c_hi rounded, e = the exact rounding error of that product (FMA), the remaining
 // cross terms are O(1e-3) turns; frac(p) is exact in fp32 (|p| < 2^22 turns, i.e. |z| < 2 m).
+// lim_v: bins |k(v)| <= lim_v are kept, the others get H = 0 (the band limit of the line, -1 if |k(u)| is outside it).
 template <bool DERIV>
-__device__ __forceinline__ void k32t_apply_h(float2 (&v)[32], const Params& p, const float2* kap_s, int lane, float c_hi, float c_lo) {
+__device__ __forceinline__ void k32t_apply_h(float2 (&v)[32], const Params& p, const float2* kap_s, int lane, float c_hi, float c_lo,
+                                             int lim_v) {
     const float MAGIC = 12582912.f;                                   // 1.5 * 2^23: round to nearest integer
 #pragma unroll
     for (int i = 0; i < 32; ++i) {
-        const int f = lane + 32 * i;
-        const float2 k = kap_s[f <= 512 ? f : 1024 - f];
+        const int f = lane + 32 * i, rf = f <= 512 ? f : 1024 - f;
+        const float2 k = kap_s[rf];
         const float pp = __fmul_rn(k.x, c_hi);
         float s = __fmaf_rn(k.x, c_hi, -pp);
         s = __fmaf_rn(k.y, c_hi, s);
@@ -103,11 +105,12 @@ __device__ __forceinline__ void k32t_apply_h(float2 (&v)[32], const Params& p, c
         const float r = __fadd_rn(__fadd_rn(pp, -kk), s);
         float sn, cn;
         __sincosf(r * 6.283185307179586f, &sn, &cn);
+        const float sc = rf <= lim_v ? p.inv_m2 : 0.f;
         if constexpr (DERIV) {
             const double kz_l = ((double)k.x + (double)k.y) * (6.283185307179586 * p.lambda);    // sqrt(1 - lambda^2 f^2)
-            v[i] = cmul_scaled(v[i], -sn, cn, (float)(kz_l - p.kshift) * p.inv_m2);
+            v[i] = cmul_scaled(v[i], -sn, cn, (float)(kz_l - p.kshift) * sc);
         } else {
-            v[i] = cmul_scaled(v[i], cn, sn, p.inv_m2);
+            v[i] = cmul_scaled(v[i], cn, sn, sc);
         }
     }
 }
@@ -229,7 +232,8 @@ k32t_rows_fwd(const Params p, const __grid_constant__ CUtensorMap tmapT, int pla
 // ---------------------------------------------------------------------------------------------------
 // pass 2: one warp per line u of the transposed workspace: FFT over y, x H, inverse FFT, in place
 // ---------------------------------------------------------------------------------------------------
-template <bool PADDED>
+// BL: band-limited calls (p.band_limit; a template parameter so that the plain instantiations stay the code they were)
+template <bool PADDED, bool BL = false>
 __global__ void __launch_bounds__(32 * K32T_LINE_WARPS, K32T_LINE_CTAS) k32t_lines(const Params p, int plane0, int nlines) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     constexpr int XCH_B = K32_LP * 8, KAP_B = KAP_STRIDE * 8;
@@ -283,6 +287,11 @@ __global__ void __launch_bounds__(32 * K32T_LINE_WARPS, K32T_LINE_CTAS) k32t_lin
         float2* row = p.ws + (size_t)line * N;
         float c_hi, c_lo;
         k32t_phase_constant(p, (plane0 + img) / p.C, &c_hi, &c_lo);
+        int lim_v = 1024;                                            // every bin
+        if constexpr (BL) {
+            const int lim = band_limit_of(p, (plane0 + img) / p.C), ul = line & 1023;
+            lim_v = (ul <= 512 ? ul : 1024 - ul) <= lim ? lim : -1;
+        }
         mbar_wait(bar, phase);
         phase ^= 1u;
         float2 v[32];
@@ -304,8 +313,8 @@ __global__ void __launch_bounds__(32 * K32T_LINE_WARPS, K32T_LINE_CTAS) k32t_lin
         __syncwarp();
         lds16<RowLayout32, 0>(v, xch + 33 * lane);
         fwd32_table(v, tw + lane);                                   // v[i] = frequency lane + 32 i
-        if (p.h_mode == H_DERIV) k32t_apply_h<true>(v, p, kap_s, lane, c_hi, c_lo);
-        else k32t_apply_h<false>(v, p, kap_s, lane, c_hi, c_lo);
+        if (p.h_mode == H_DERIV) k32t_apply_h<true>(v, p, kap_s, lane, c_hi, c_lo, lim_v);
+        else k32t_apply_h<false>(v, p, kap_s, lane, c_hi, c_lo, lim_v);
         inv32_first(v);
         __syncwarp();                                                // every lane has read its exchange values
         sts16<RowLayout32, 0>(v, xch + 33 * lane);

@@ -313,7 +313,9 @@ __device__ __forceinline__ void k64_stage_kz(double* kz_s, const double* kzt, in
 
 // PAIRS: the kappa slab holds fp32 (hi, lo) pairs and t = c kappa is formed in double-float fp32 (no fp64, no F2F; see
 // k32t_apply_h); otherwise fp64 entries (the table of the generic row kernels' column order).
-template <bool PADDED, bool PAIRS>
+// BL: band-limited calls (p.band_limit).  A template parameter here, not a runtime test as in the other column kernels:
+// the padded kernel is at its register limit, and the plain instantiations stay the code they were.
+template <bool PADDED, bool PAIRS, bool BL = false>
 __global__ void __launch_bounds__(64 * K64_CC, 2) k64_cols(const Params p, int plane0, int nimg) {
     constexpr int L = K64_L, CC = K64_CC, nslab = L / CC;
     using LAY = ColLayout32<CC>;
@@ -369,6 +371,14 @@ __global__ void __launch_bounds__(64 * K64_CC, 2) k64_cols(const Params p, int p
         }
         __syncthreads();                                             // the dense rows are consumed
         const double cph = phase_constant_of(p, plane / p.C);
+        // band limit: column col0 + c holds frequency v (split order with the warp-pair row kernels, digit-reversed
+        // otherwise); rows |k(u)| <= lim_u are kept if |k(v)| is within the limit, none otherwise
+        int lim_u = L;
+        if constexpr (BL) {
+            const int vpos = PAIRS ? 2 * ((col0 + c) & 1023) + ((col0 + c) >> 10) : freq_of_pos(11, col0 + c);
+            const int lim = band_limit_of(p, plane / p.C);
+            lim_u = (vpos <= L / 2 ? vpos : L - vpos) <= lim ? lim : -1;
+        }
         // ---- forward 1024-point transform of this half ----
         if (h == 1) k64_twiddle64<-1>(v);
         fwd32_first(v);
@@ -395,11 +405,12 @@ __global__ void __launch_bounds__(64 * K64_CC, 2) k64_cols(const Params p, int p
                 const float r = __fadd_rn(__fadd_rn(pp, -kk), sacc);
                 float sn, cn;
                 __sincosf(r * 6.283185307179586f, &sn, &cn);
+                const float sc = ru <= lim_u ? p.inv_m2 : 0.f;       // H = 0 outside the band limit
                 if (p.h_mode == H_DERIV) {
                     const double kz_l = ((double)k.x + (double)k.y) * (6.283185307179586 * p.lambda);
-                    v[i] = cmul_scaled(v[i], -sn, cn, (float)(kz_l - p.kshift) * p.inv_m2);
+                    v[i] = cmul_scaled(v[i], -sn, cn, (float)(kz_l - p.kshift) * sc);
                 } else {
-                    v[i] = cmul_scaled(v[i], cn, sn, p.inv_m2);
+                    v[i] = cmul_scaled(v[i], cn, sn, sc);
                 }
             }
         } else {
@@ -413,8 +424,9 @@ __global__ void __launch_bounds__(64 * K64_CC, 2) k64_cols(const Params p, int p
                 const double rr = tt - __dadd_rn(__dadd_rn(tt, MAGIC), -MAGIC);
                 float sn, cn;
                 __sincosf((float)rr * 6.283185307179586f, &sn, &cn);
-                if (p.h_mode == H_DERIV) v[i] = cmul_scaled(v[i], -sn, cn, (float)(kap * k2pl - p.kshift) * p.inv_m2);
-                else v[i] = cmul_scaled(v[i], cn, sn, p.inv_m2);
+                const float sc = ru <= lim_u ? p.inv_m2 : 0.f;       // H = 0 outside the band limit
+                if (p.h_mode == H_DERIV) v[i] = cmul_scaled(v[i], -sn, cn, (float)(kap * k2pl - p.kshift) * sc);
+                else v[i] = cmul_scaled(v[i], cn, sn, sc);
             }
         }
         // ---- inverse 1024-point transform of this half ----

@@ -14,7 +14,7 @@ from typing import Optional, Sequence, Tuple, Union
 import torch
 
 from . import _lib as L
-from .functional import _c64, _f32, _ptr, _stream
+from .functional import _c64, _entry, _f32, _ptr, _stream
 
 _OUT_MODES = {"intensity": L.OUT_INTENSITY, "complex": L.OUT_COMPLEX, "abs_angle": L.OUT_ABS_ANGLE, None: None}
 
@@ -38,7 +38,7 @@ def _stack_distances(z, b: int, device: torch.device) -> Tuple[torch.Tensor, int
 
 def focal_stack(x: torch.Tensor, z: Union[torch.Tensor, Sequence[float]], wavelength: float, pixel_size: float,
                 zero_padding: bool = False, *, hologram: bool = False, output: Optional[str] = "intensity",
-                moments: bool = False):
+                moments: bool = False, band_limit: bool = False):
     """Propagate every sample of ``x`` to K distances.
 
     x: [B, 1, N, N] or [B, N, N]; complex64 field, real field, or (``hologram=True``) an intensity whose square root is
@@ -46,6 +46,7 @@ def focal_stack(x: torch.Tensor, z: Union[torch.Tensor, Sequence[float]], wavele
     z: [K] or [B, K] distances in metres.
     output: "intensity" (fp32 [B, K, N, N]), "complex" (complex64), "abs_angle" (tuple of fp32 |U|, angle(U)) or None.
     moments: also return the float64 [B, K, 3] moments (Sum |U|, Sum |U|^2, Sum |U|^4) over each N x N plane.
+    band_limit: band-limited transfer function (``ASM(..., band_limit=True)``), the limit taken from each plane's own z.
     Returns the images, ``(images, moments)``, or only the moments when ``output`` is None.
     """
     if output not in _OUT_MODES:
@@ -91,9 +92,10 @@ def focal_stack(x: torch.Tensor, z: Union[torch.Tensor, Sequence[float]], wavele
             out1 = torch.empty((b, k, n, n), dtype=torch.float32, device=dev)
     mom = torch.empty((b, k, 3), dtype=torch.float64, device=dev) if moments else None
     with torch.cuda.device(dev):
-        rc = lib.asm_b200_focal_stack(_ptr(xin), None, _ptr(zt), zd, k, _ptr(out0), _ptr(out1), _ptr(mom), b, n,
-                                      int(zero_padding), in_mode, L.OUT_INTENSITY if out_mode is None else out_mode,
-                                      float(wavelength), float(pixel_size), 1.0, _ptr(ws), ws.numel(), _stream())
+        fn, bl = _entry("asm_b200_focal_stack", band_limit)
+        rc = fn(_ptr(xin), None, _ptr(zt), zd, k, _ptr(out0), _ptr(out1), _ptr(mom), b, n, int(zero_padding), in_mode,
+                L.OUT_INTENSITY if out_mode is None else out_mode, float(wavelength), float(pixel_size), 1.0, _ptr(ws),
+                ws.numel(), _stream(), *bl)
     L.check(rc)
     images = (out0, out1) if output == "abs_angle" else out0
     if output is None:
@@ -118,7 +120,8 @@ def focus_metric(moments: torch.Tensor, n_pixels: int, metric: str = "tamura") -
 
 
 def autofocus(x: torch.Tensor, z: Union[torch.Tensor, Sequence[float]], wavelength: float, pixel_size: float,
-              zero_padding: bool = False, *, hologram: bool = True, metric: str = "tamura", select: str = "min"):
+              zero_padding: bool = False, *, hologram: bool = True, metric: str = "tamura", select: str = "min",
+              band_limit: bool = False):
     """Pick, per sample, the candidate distance whose plane is extreme in ``metric``.
 
     One moments-only focal stack: no [B, K, N, N] tensor is allocated.  ``select`` is "min" or "max": a pure-phase
@@ -128,7 +131,8 @@ def autofocus(x: torch.Tensor, z: Union[torch.Tensor, Sequence[float]], waveleng
     """
     if select not in ("min", "max"):
         raise ValueError(f"select must be 'min' or 'max'; got {select!r}")
-    mom = focal_stack(x, z, wavelength, pixel_size, zero_padding, hologram=hologram, output=None, moments=True)
+    mom = focal_stack(x, z, wavelength, pixel_size, zero_padding, hologram=hologram, output=None, moments=True,
+                      band_limit=band_limit)
     n = x.shape[-1]
     curve = focus_metric(mom, n * n, metric)
     index = torch.argmin(curve, dim=1) if select == "min" else torch.argmax(curve, dim=1)

@@ -74,31 +74,47 @@ def _workspace(b: int, c: int, n: int, pad: bool, device: torch.device) -> torch
     return torch.empty(nbytes, dtype=torch.uint8, device=device)
 
 
-def _forward_call(in0, in1, z, zd, out0, out1, b, c, n, pad, in_mode, out_mode, lamb, px, in_scale, out_scale):
+# band_limit=True: the band-limited transfer function of include/asm_b200.h (asm_b200_*_bl): bins outside
+# |f_x|, |f_y| <= 1 / (lambda sqrt(1 + (2 z / (M px))^2)) get H = 0 (Matsushima & Shimobaba 2009).  Opt-in everywhere;
+# without it the plain entry point is called, exactly as before the option existed.
+def _entry(name: str, band_limit: bool):
+    """(C function, trailing arguments): the plain entry point, or its _bl variant with band_limit = 1."""
+    lib = L.load()
+    if not band_limit:
+        return getattr(lib, name), ()
+    if not hasattr(lib, name + "_bl"):
+        raise L.AsmB200Error(f"{L.LIB_PATH} has no {name}_bl: rebuild it (band_limit=True needs the band-limited entry points)")
+    return getattr(lib, name + "_bl"), (1,)
+
+
+def _forward_call(in0, in1, z, zd, out0, out1, b, c, n, pad, in_mode, out_mode, lamb, px, in_scale, out_scale,
+                  band_limit=False):
     ws = _workspace(b, c, n, pad, in0.device)
     with torch.cuda.device(in0.device):
-        rc = L.load().asm_b200_forward(_ptr(in0), _ptr(in1), _ptr(z), zd, _ptr(out0), _ptr(out1), b, c, n, int(pad),
-                                       in_mode, out_mode, float(lamb), float(px), float(in_scale), float(out_scale),
-                                       _ptr(ws), ws.numel(), _stream())
+        fn, bl = _entry("asm_b200_forward", band_limit)
+        rc = fn(_ptr(in0), _ptr(in1), _ptr(z), zd, _ptr(out0), _ptr(out1), b, c, n, int(pad), in_mode, out_mode,
+                float(lamb), float(px), float(in_scale), float(out_scale), _ptr(ws), ws.numel(), _stream(), *bl)
     L.check(rc)
 
 
-def _adjoint_call(in0, in1, z, zd, aux0, aux1, out0, out1, b, c, n, pad, in_mode, out_mode, lamb, px, in_scale):
+def _adjoint_call(in0, in1, z, zd, aux0, aux1, out0, out1, b, c, n, pad, in_mode, out_mode, lamb, px, in_scale,
+                  band_limit=False):
     ws = _workspace(b, c, n, pad, in0.device)
     with torch.cuda.device(in0.device):
-        rc = L.load().asm_b200_adjoint(_ptr(in0), _ptr(in1), _ptr(z), zd, _ptr(aux0), _ptr(aux1), _ptr(out0), _ptr(out1),
-                                       b, c, n, int(pad), in_mode, out_mode, float(lamb), float(px), float(in_scale),
-                                       _ptr(ws), ws.numel(), _stream())
+        fn, bl = _entry("asm_b200_adjoint", band_limit)
+        rc = fn(_ptr(in0), _ptr(in1), _ptr(z), zd, _ptr(aux0), _ptr(aux1), _ptr(out0), _ptr(out1), b, c, n, int(pad),
+                in_mode, out_mode, float(lamb), float(px), float(in_scale), _ptr(ws), ws.numel(), _stream(), *bl)
     L.check(rc)
 
 
-def _grad_z_call(in0, in1, z, zd, cot0, cot1, cot_mode, b, c, n, pad, in_mode, lamb, px, in_scale) -> torch.Tensor:
+def _grad_z_call(in0, in1, z, zd, cot0, cot1, cot_mode, b, c, n, pad, in_mode, lamb, px, in_scale,
+                 band_limit=False) -> torch.Tensor:
     ws = _workspace(b, c, n, pad, in0.device)
     gz = torch.empty(b, dtype=torch.float64, device=in0.device)
     with torch.cuda.device(in0.device):
-        rc = L.load().asm_b200_grad_z(_ptr(in0), _ptr(in1), _ptr(z), zd, _ptr(cot0), _ptr(cot1), cot_mode, _ptr(gz),
-                                      b, c, n, int(pad), in_mode, float(lamb), float(px), float(in_scale),
-                                      _ptr(ws), ws.numel(), _stream())
+        fn, bl = _entry("asm_b200_grad_z", band_limit)
+        rc = fn(_ptr(in0), _ptr(in1), _ptr(z), zd, _ptr(cot0), _ptr(cot1), cot_mode, _ptr(gz), b, c, n, int(pad),
+                in_mode, float(lamb), float(px), float(in_scale), _ptr(ws), ws.numel(), _stream(), *bl)
     L.check(rc)
     return gz
 
@@ -148,7 +164,7 @@ def _grad_like(g: torch.Tensor, z_meta) -> Optional[torch.Tensor]:
 # raw (non-differentiable) entry points -- also what bench.py times
 # ---------------------------------------------------------------------------------------------------
 def asm_forward_raw(field: torch.Tensor, z, lamb: float, px: float, pad: bool, out_mode: int = L.OUT_COMPLEX,
-                    out: Optional[torch.Tensor] = None) -> torch.Tensor:
+                    out: Optional[torch.Tensor] = None, band_limit: bool = False) -> torch.Tensor:
     """complex64 (or real fp32) [B,C,N,N] -> complex64 field or fp32 intensity, one fused pipeline."""
     b, c, n = _check_field(field, "O")
     if field.is_complex():
@@ -159,18 +175,20 @@ def asm_forward_raw(field: torch.Tensor, z, lamb: float, px: float, pad: bool, o
     if out is None:
         out = torch.empty((b, c, n, n), device=x.device,
                           dtype=torch.complex64 if out_mode == L.OUT_COMPLEX else torch.float32)
-    _forward_call(x, None, zt, zd, out, None, b, c, n, pad, in_mode, out_mode, lamb, px, 1.0, 1.0)
+    _forward_call(x, None, zt, zd, out, None, b, c, n, pad, in_mode, out_mode, lamb, px, 1.0, 1.0, band_limit)
     return out
 
 
-def asm_adjoint_raw(g: torch.Tensor, z, lamb: float, px: float, pad: bool, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+def asm_adjoint_raw(g: torch.Tensor, z, lamb: float, px: float, pad: bool, out: Optional[torch.Tensor] = None,
+                    band_limit: bool = False) -> torch.Tensor:
     """Adjoint propagation of a complex64 cotangent (exact VJP of ASM w.r.t. O)."""
     b, c, n = _check_field(g, "cotangent")
     x = _c64(g)
     zt, zd = prepare_distance(z, b, x.device)
     if out is None:
         out = torch.empty_like(x)
-    _adjoint_call(x, None, zt, zd, None, None, out, None, b, c, n, pad, L.IN_COMPLEX, L.OUT_COMPLEX, lamb, px, 1.0)
+    _adjoint_call(x, None, zt, zd, None, None, out, None, b, c, n, pad, L.IN_COMPLEX, L.OUT_COMPLEX, lamb, px, 1.0,
+                  band_limit)
     return out
 
 
@@ -181,7 +199,7 @@ class AsmPropagate(torch.autograd.Function):
     """U = ASM(O, lamb, z, px, zero_padding)  -- complex64 out (the reference returns complex128)."""
 
     @staticmethod
-    def forward(ctx, field, z, lamb, px, pad):
+    def forward(ctx, field, z, lamb, px, pad, band_limit=False):
         b, c, n = _check_field(field, "O")
         if field.is_complex():
             x, in_mode = _c64(field), L.IN_COMPLEX
@@ -189,60 +207,63 @@ class AsmPropagate(torch.autograd.Function):
             x, in_mode = _f32(field), L.IN_REAL
         zt, zd = prepare_distance(z, b, x.device)
         out = torch.empty((b, c, n, n), dtype=torch.complex64, device=x.device)
-        _forward_call(x, None, zt, zd, out, None, b, c, n, pad, in_mode, L.OUT_COMPLEX, lamb, px, 1.0, 1.0)
+        _forward_call(x, None, zt, zd, out, None, b, c, n, pad, in_mode, L.OUT_COMPLEX, lamb, px, 1.0, 1.0, band_limit)
         z_meta = _z_meta(z)
         need_z = z_meta is not None and ctx.needs_input_grad[1]
         ctx.save_for_backward(x if need_z else None, zt)      # the field is only needed for the distance gradient
-        ctx.meta = (b, c, n, bool(pad), float(lamb), float(px), zd, in_mode, field.dtype, z_meta)
+        ctx.meta = (b, c, n, bool(pad), float(lamb), float(px), zd, in_mode, field.dtype, z_meta, bool(band_limit))
         return out
 
     @staticmethod
     def backward(ctx, grad_out):
         x, zt = ctx.saved_tensors
-        b, c, n, pad, lamb, px, zd, in_mode, in_dtype, z_meta = ctx.meta
+        b, c, n, pad, lamb, px, zd, in_mode, in_dtype, z_meta, bl = ctx.meta
         g = _c64(grad_out)
         grad_field = grad_z = None
         if ctx.needs_input_grad[0]:
             go = torch.empty_like(g)
-            _adjoint_call(g, None, zt, zd, None, None, go, None, b, c, n, pad, L.IN_COMPLEX, L.OUT_COMPLEX, lamb, px, 1.0)
+            _adjoint_call(g, None, zt, zd, None, None, go, None, b, c, n, pad, L.IN_COMPLEX, L.OUT_COMPLEX, lamb, px, 1.0,
+                          bl)
             grad_field = go.to(in_dtype) if in_dtype.is_complex else go.real.to(in_dtype)
         if ctx.needs_input_grad[1] and z_meta is not None and x is not None:
-            gz = _grad_z_call(x, None, zt, zd, g, None, L.IN_COMPLEX, b, c, n, pad, in_mode, lamb, px, 1.0)
+            gz = _grad_z_call(x, None, zt, zd, g, None, L.IN_COMPLEX, b, c, n, pad, in_mode, lamb, px, 1.0, bl)
             grad_z = _grad_like(gz, z_meta)
-        return grad_field, grad_z, None, None, None
+        return grad_field, grad_z, None, None, None, None
 
 
 class HoloField(torch.autograd.Function):
     """U = ASM(A exp(i phase pn), z, zero_padding=True) as complex64 (utils/Forward_model.py:20-24)."""
 
     @staticmethod
-    def forward(ctx, amplitude, phase, z, lamb, px, phase_normalize, pad):
+    def forward(ctx, amplitude, phase, z, lamb, px, phase_normalize, pad, band_limit=False):
         b, c, n = _check_field(phase, "phase")
         a, ph, in_mode = _amp_phase(amplitude, phase)
         zt, zd = prepare_distance(z, b, ph.device)
         out = torch.empty((b, c, n, n), dtype=torch.complex64, device=ph.device)
-        _forward_call(a, ph, zt, zd, out, None, b, c, n, pad, in_mode, L.OUT_COMPLEX, lamb, px, phase_normalize, 1.0)
+        _forward_call(a, ph, zt, zd, out, None, b, c, n, pad, in_mode, L.OUT_COMPLEX, lamb, px, phase_normalize, 1.0,
+                      band_limit)
         ctx.save_for_backward(a, ph, zt)
         ctx.meta = (b, c, n, bool(pad), float(lamb), float(px), zd, float(phase_normalize), amplitude.dtype, phase.dtype,
-                    _z_meta(z), in_mode, tuple(amplitude.shape))
+                    _z_meta(z), in_mode, tuple(amplitude.shape), bool(band_limit))
         return out
 
     @staticmethod
     def backward(ctx, grad_out):
         a, ph, zt = ctx.saved_tensors
-        b, c, n, pad, lamb, px, zd, pn, adt, pdt, z_meta, in_mode, ashape = ctx.meta
+        b, c, n, pad, lamb, px, zd, pn, adt, pdt, z_meta, in_mode, ashape, bl = ctx.meta
         g = _c64(grad_out)
         ga = gp = gz = None
         if ctx.needs_input_grad[0] or ctx.needs_input_grad[1]:
             af = a if in_mode == L.IN_AMP_PHASE else a.expand(ph.shape).contiguous()
             ga = torch.empty_like(af)
             gp = torch.empty_like(ph)
-            _adjoint_call(g, None, zt, zd, af, ph, ga, gp, b, c, n, pad, L.IN_COMPLEX, L.OUT_GRAD_AP, lamb, px, pn)
+            _adjoint_call(g, None, zt, zd, af, ph, ga, gp, b, c, n, pad, L.IN_COMPLEX, L.OUT_GRAD_AP, lamb, px, pn, bl)
             ga = (ga if in_mode == L.IN_AMP_PHASE else ga.sum().reshape(ashape)).to(adt)
             gp = gp.to(pdt)
         if ctx.needs_input_grad[2] and z_meta is not None:
-            gz = _grad_like(_grad_z_call(a, ph, zt, zd, g, None, L.IN_COMPLEX, b, c, n, pad, in_mode, lamb, px, pn), z_meta)
-        return ga, gp, gz, None, None, None, None
+            gz = _grad_like(_grad_z_call(a, ph, zt, zd, g, None, L.IN_COMPLEX, b, c, n, pad, in_mode, lamb, px, pn, bl),
+                            z_meta)
+        return ga, gp, gz, None, None, None, None, None
 
 
 class HoloIntensity(torch.autograd.Function):
@@ -253,53 +274,56 @@ class HoloIntensity(torch.autograd.Function):
     """
 
     @staticmethod
-    def forward(ctx, amplitude, phase, z, lamb, px, phase_normalize, pad):
+    def forward(ctx, amplitude, phase, z, lamb, px, phase_normalize, pad, band_limit=False):
         b, c, n = _check_field(phase, "phase")
         a, ph, in_mode = _amp_phase(amplitude, phase)
         zt, zd = prepare_distance(z, b, ph.device)
         need = any(ctx.needs_input_grad[:3])
         out = torch.empty((b, c, n, n), dtype=torch.float32, device=ph.device)
         u = torch.empty((b, c, n, n), dtype=torch.complex64, device=ph.device) if need else None
-        _forward_call(a, ph, zt, zd, out, u, b, c, n, pad, in_mode, L.OUT_INTENSITY, lamb, px, phase_normalize, 1.0)
+        _forward_call(a, ph, zt, zd, out, u, b, c, n, pad, in_mode, L.OUT_INTENSITY, lamb, px, phase_normalize, 1.0,
+                      band_limit)
         if need:
             ctx.save_for_backward(a, ph, zt, u)
         ctx.meta = (b, c, n, bool(pad), float(lamb), float(px), zd, float(phase_normalize), amplitude.dtype, phase.dtype,
-                    _z_meta(z), in_mode, tuple(amplitude.shape))
+                    _z_meta(z), in_mode, tuple(amplitude.shape), bool(band_limit))
         return out
 
     @staticmethod
     def backward(ctx, grad_out):
         a, ph, zt, u = ctx.saved_tensors
-        b, c, n, pad, lamb, px, zd, pn, adt, pdt, z_meta, in_mode, ashape = ctx.meta
+        b, c, n, pad, lamb, px, zd, pn, adt, pdt, z_meta, in_mode, ashape, bl = ctx.meta
         w = _f32(grad_out)
         ga = gp = gz = None
         if ctx.needs_input_grad[0] or ctx.needs_input_grad[1]:
             af = a if in_mode == L.IN_AMP_PHASE else a.expand(ph.shape).contiguous()
             ga = torch.empty_like(af)
             gp = torch.empty_like(ph)
-            _adjoint_call(w, u, zt, zd, af, ph, ga, gp, b, c, n, pad, L.IN_COT_FIELD, L.OUT_GRAD_AP, lamb, px, pn)
+            _adjoint_call(w, u, zt, zd, af, ph, ga, gp, b, c, n, pad, L.IN_COT_FIELD, L.OUT_GRAD_AP, lamb, px, pn, bl)
             ga = (ga if in_mode == L.IN_AMP_PHASE else ga.sum().reshape(ashape)).to(adt)
             gp = gp.to(pdt)
         if ctx.needs_input_grad[2] and z_meta is not None:
-            gz = _grad_like(_grad_z_call(a, ph, zt, zd, w, u, L.IN_COT_FIELD, b, c, n, pad, in_mode, lamb, px, pn), z_meta)
-        return ga, gp, gz, None, None, None, None
+            gz = _grad_like(_grad_z_call(a, ph, zt, zd, w, u, L.IN_COT_FIELD, b, c, n, pad, in_mode, lamb, px, pn, bl),
+                            z_meta)
+        return ga, gp, gz, None, None, None, None, None
 
 
 # ---------------------------------------------------------------------------------------------------
 # fused no-grad fast paths
 # ---------------------------------------------------------------------------------------------------
-def holo_abs_angle(amplitude, phase, z, lamb, px, phase_normalize, pad=True):
+def holo_abs_angle(amplitude, phase, z, lamb, px, phase_normalize, pad=True, band_limit=False):
     """(|U|, angle U) in one pipeline (utils/Forward_model.py:27-34), no autograd graph."""
     b, c, n = _check_field(phase, "phase")
     a, ph, in_mode = _amp_phase(amplitude, phase)
     zt, zd = prepare_distance(z, b, ph.device)
     amp = torch.empty((b, c, n, n), dtype=torch.float32, device=ph.device)
     ang = torch.empty_like(amp)
-    _forward_call(a, ph, zt, zd, amp, ang, b, c, n, pad, in_mode, L.OUT_ABS_ANGLE, lamb, px, phase_normalize, 1.0)
+    _forward_call(a, ph, zt, zd, amp, ang, b, c, n, pad, in_mode, L.OUT_ABS_ANGLE, lamb, px, phase_normalize, 1.0,
+                  band_limit)
     return amp, ang
 
 
-def holo_intensity_pair(amplitude, phase_a, phase_b, z_a, z_b, lamb, px, phase_normalize, pad=True):
+def holo_intensity_pair(amplitude, phase_a, phase_b, z_a, z_b, lamb, px, phase_normalize, pad=True, band_limit=False):
     """Two no-grad intensity syntheses sharing one amplitude (utils/Data_loader.py:31-32) written into ONE [2B,C,N,N]
     output allocation, without concatenating the inputs: each phase tensor is read in place."""
     b, c, n = _check_field(phase_a, "phase")
@@ -308,11 +332,11 @@ def holo_intensity_pair(amplitude, phase_a, phase_b, z_a, z_b, lamb, px, phase_n
         a, ph, in_mode = _amp_phase(amplitude, ph_k)
         zt, zd = prepare_distance(z_k, b, ph.device)
         _forward_call(a, ph, zt, zd, out[k * b:(k + 1) * b], None, b, c, n, pad, in_mode, L.OUT_INTENSITY, lamb, px,
-                      phase_normalize, 1.0)
+                      phase_normalize, 1.0, band_limit)
     return out[:b], out[b:]
 
 
-def back_prop_fused(holo, z, lamb, px, amplitude_normalize, amp_pha: bool):
+def back_prop_fused(holo, z, lamb, px, amplitude_normalize, amp_pha: bool, band_limit: bool = False):
     """cat(|s U|, angle(s U)) or cat(re, im) * s of U = ASM(sqrt(holo), z) in one pipeline
     (utils/Forward_model.py:55-65), fp32 [B,2,N,N]."""
     b, c, n = _check_field(holo, "holo")
@@ -324,7 +348,7 @@ def back_prop_fused(holo, z, lamb, px, amplitude_normalize, amp_pha: bool):
     zt, zd = prepare_distance(z, b, h.device)
     out = torch.empty((b, 2, n, n), dtype=torch.float32, device=h.device)
     _forward_call(h, None, zt, zd, out, None, b, 1, n, False, L.IN_SQRT_REAL,
-                  L.OUT_ABSANG_CAT if amp_pha else L.OUT_REIM_CAT, lamb, px, 1.0, amplitude_normalize)
+                  L.OUT_ABSANG_CAT if amp_pha else L.OUT_REIM_CAT, lamb, px, 1.0, amplitude_normalize, band_limit)
     return out
 
 
